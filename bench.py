@@ -3,6 +3,7 @@
 insertPointCloud of one synthetic scan of the named shape).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4] [--impl reference]
+                    [--dump-outputs DIR]
 
 Default = BASELINE configs[1] ("config 2": OccupancyMap 2 cm, 131 072-point Velodyne-64-shaped
 scan stream, max_range 30 m), the configuration the metric is quoted on; --config 3 (colour map,
@@ -27,6 +28,10 @@ configurations the same way.
            ceiling (tools/atomic_ceiling.cu -> profiles/r02_atomic_ceiling.jsonl).
 * cpu_baseline / --impl reference: the unmodified reference (oracle/_ref/libufo_ref.so) on a bounded
            sample of the same workload on the host cores.
+* --dump-outputs DIR: after the timed steps of `value`, the map they built (voxel keys f64, log-odds
+           f32, colour f32; a fixed hash sample above 2^20 voxels) and the last scan's counters, as
+           DIR/<name>.npy.  The scans are seeded, so the same arguments feed the same inputs and two
+           builds can be compared output for output.
 
 Multi-GPU (torchrun, one rank per GPU): --mode route (default) = ONE scan stream, rays split over
 the GPUs, state owned by space, marks forwarded over NVLink peer memory; --mode merge = one sensor
@@ -359,6 +364,38 @@ def cpu_baseline_sample(cfg, origins, xyzs, rgbs):
                       "async=false, 1 caller + 1 hit thread of %d host cores" % (stride, npts, os.cpu_count() or 0)}
 
 
+DUMP_MAX_VOXELS = 1 << 20   # 40 B a voxel at most (keys f64, log-odds f32, colour f32): 40 MB
+COUNTER_NAMES = ("points", "rays", "touched_voxels", "hit_voxels", "touched_octets", "touched_lines",
+                 "touched_blocks", "touched_d3", "touched_bricks", "upper_nodes", "blocks_in_map", "bricks_in_map")
+
+
+def dump_outputs(out_dir, m, color, prefix=""):
+    """What the timed insert path leaves a caller: the map's value field (every voxel with a
+    non-default payload) and the result counters of the last scan, as .npy files in `out_dir`.
+    A field of more than DUMP_MAX_VOXELS voxels is sampled by a fixed hash of the voxel code, so
+    two builds that computed the same field write the same sample."""
+    os.makedirs(out_dir, exist_ok=True)
+    m.wait()
+    codes, occ, rgb = m.value_field(sort=False)
+    if len(codes) > DUMP_MAX_VOXELS:
+        mixed = codes * np.uint64(0x9E3779B97F4A7C15)   # wraps: a fixed bijective hash of the code
+        keep = mixed < np.uint64(int(2.0 ** 64 * DUMP_MAX_VOXELS / len(codes)))
+        codes, occ, rgb = codes[keep], occ[keep], rgb[keep]
+    order = np.argsort(codes, kind="stable")
+    codes, occ, rgb = codes[order], occ[order], rgb[order]
+    keys = np.zeros((len(codes), 3), np.float64)   # the depth-0 key: code bits interleaved x, y, z
+    for i in range(21):
+        for a in range(3):
+            keys[:, a] += ((codes >> np.uint64(3 * i + a)) & np.uint64(1)).astype(np.float64) * float(1 << i)
+    st = m.stats()
+    arrays = {"voxel_keys": keys, "log_odds": occ.astype(np.float32),
+              "scan_counters": np.array([float(st[k]) for k in COUNTER_NAMES], np.float64)}
+    if color:
+        arrays["rgb"] = rgb.astype(np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -376,6 +413,9 @@ def main():
                          "(BASELINE config #5, weak scaling); 'sensors' = independent replicas (one sensor stream + "
                          "map per GPU, no merge); 'shard' = one stream broadcast, every GPU walks every ray and "
                          "keeps its own bricks (variant 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of `value`, write the map's value field (sampled above %d voxels) "
+                         "and the last scan's counters to DIR/<name>.npy" % DUMP_MAX_VOXELS)
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     cfg = CONFIGS[args.config]
@@ -509,6 +549,8 @@ def main():
     for k in range(args.warmup):
         feed_device(m, k)
     ms_dev, per_scan, launches, clocks = timed_loop(m, feed_device, args.warmup, args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, m, cfg["color"], "rank%d_" % rank if world > 1 else "")
     dev_bytes = per_scan[-1]["device_bytes"]
     # one more scan with visit / mark counting switched on (not timed): raycast counters
     m.set_profiling(2)

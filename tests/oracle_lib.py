@@ -1,17 +1,25 @@
 """ctypes wrappers for the two CPU checkers (TEST INFRASTRUCTURE ONLY).
 
 * ``RefMap``    -> oracle/_ref/libufo_ref.so   (the unmodified reference, see
-                  oracle/ref_harness.cpp); available wherever the prebuilt .so
-                  travelled or /root/reference is mounted.
+                  oracle/ref_harness.cpp) where it has been built; elsewhere the
+                  restatement below, every answer checked against the digest of
+                  the reference's answer to the same question after the same
+                  history (tests/golden/reference/answers.npz).  Regenerate that
+                  ledger with the reference built: delete it, then run the whole
+                  suite with UFO_REFERENCE_RECORD=<repo>/tests/golden/reference/answers.npz.
 * ``OracleMap`` -> oracle/libufo_oracle.so     (plain-C restatement, oracle/ufo_oracle.c)
 
 Both expose the same methods; state is compared as a *value field*
 (``value_field()``: every depth-0 voxel with a non-default payload), never as
 tree shape (SURVEY.md Appendix A.7).
 """
+import atexit
 import ctypes as C
+import functools
+import hashlib
 import os
 import subprocess
+import threading
 
 import numpy as np
 
@@ -19,6 +27,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 REF_SO = os.path.join(ORACLE_DIR, "_ref", "libufo_ref.so")
 ORACLE_SO = os.path.join(ORACLE_DIR, "libufo_oracle.so")
+LEDGER = os.path.join(ROOT, "tests", "golden", "reference", "answers.npz")
 
 DEFAULT_MODEL = dict(occupied_thres=0.5, free_thres=0.5, prob_hit=0.7, prob_miss=0.4,
                      clamping_thres_min=0.1192, clamping_thres_max=0.971)
@@ -280,10 +289,174 @@ class _CpuMap:
         return buf.tobytes()
 
 
+def _feed(h, value):
+    """Canonical encoding of a (nested) call argument or answer into a hash."""
+    if isinstance(value, (tuple, list)):
+        h.update(b"(%d" % len(value))
+        for v in value:
+            _feed(h, v)
+        h.update(b")")
+    elif isinstance(value, dict):
+        _feed(h, sorted(value.items()))
+    elif isinstance(value, (bytes, bytearray)):
+        h.update(b"B%d:" % len(value))
+        h.update(value)
+    elif value is None or isinstance(value, str):
+        h.update(repr(value).encode())
+    else:
+        a = np.ascontiguousarray(value)
+        h.update(("A%s%s:" % (a.dtype.str, a.shape)).encode())
+        h.update(a.tobytes())
+
+
+def _digest(*values):
+    """64-bit SHA-256 prefix of the canonical encoding of `values`."""
+    h = hashlib.sha256()
+    _feed(h, values)
+    return int.from_bytes(h.digest()[:8], "little")
+
+
+class _Answers:
+    """The reference's answers to questions asked of a map after a given history.
+
+    tests/golden/reference/answers.npz holds ``answers``: the sorted 64-bit digests of every
+    (construction, history of state changes, question, answer) the reference was seen to give.
+    With UFO_REFERENCE_RECORD=<path> every answer the compiled reference gives is added to the
+    ledger at <path> when the process exits."""
+
+    def __init__(self):
+        self._ledger = None
+        self._new = set()
+        self._lock = threading.Lock()
+
+    def ledger(self):
+        if self._ledger is None:
+            self._ledger = _read_ledger(LEDGER)
+        return self._ledger
+
+    def record(self, entry):
+        with self._lock:
+            if not self._new:
+                atexit.register(self._flush)
+            self._new.add(entry)
+
+    def _flush(self):
+        path = os.environ["UFO_REFERENCE_RECORD"]
+        answers = np.union1d(_read_ledger(path), np.array(sorted(self._new), np.uint64))
+        np.savez_compressed(path, answers=answers)
+
+
+def _read_ledger(path):
+    if not os.path.exists(path):
+        return np.empty(0, np.uint64)
+    with np.load(path) as z:
+        return z["answers"]
+
+
+_ANSWERS = _Answers()
+
+
+def _ask(real, state, question, args, compute):
+    """The reference's answer to `question(args)` on the map whose history hashes to `state`.
+
+    `compute` runs on the compiled reference when `real` (and its answer is recorded when
+    UFO_REFERENCE_RECORD is set), otherwise on the C restatement, whose answer must then be
+    the one the reference gave to the same question."""
+    answer = compute()
+    entry = _digest(_digest(state, question, args), _digest(answer))
+    if real:
+        if os.environ.get("UFO_REFERENCE_RECORD"):
+            _ANSWERS.record(entry)
+        return answer
+    answers = _ANSWERS.ledger()
+    i = np.searchsorted(answers, np.uint64(entry))
+    assert i < len(answers) and answers[i] == entry, (
+        "the C restatement's answer to %s is not one the reference gave on this history" % question)
+    return answer
+
+
+def ref_pose_from_rpy(*xyzrpy):
+    """The reference's Pose6(x, y, z, roll, pitch, yaw) as (x, y, z, qw, qx, qy, qz)."""
+    def compute():
+        out = np.empty(7)
+        _load(REF_SO if have_ref() else ORACLE_SO,
+              "ufo_ref_" if have_ref() else "ufo_oracle_")["pose_from_rpy"](*xyzrpy, out.ctypes.data)
+        return out
+    return _ask(have_ref(), b"", "pose_from_rpy", [float(v) for v in xyzrpy], compute)
+
+
+def ref_transform(pose, pts):
+    """The reference's PointCloud::transform of float64 points by a pose of ref_pose_from_rpy."""
+    pose, pts = _f64(pose), _f64(pts)
+
+    def compute():
+        out = np.empty_like(pts)
+        _load(REF_SO if have_ref() else ORACLE_SO,
+              "ufo_ref_" if have_ref() else "ufo_oracle_")["transform"](pose.ctypes.data, pts.ctypes.data,
+                                                                         len(pts), out.ctypes.data)
+        return out
+    return _ask(have_ref(), b"", "transform", [pose, pts], compute)
+
+
+def _asked(stand_in=None):
+    """Route a RefMap query through _ask (see there).  `stand_in` names the method that answers
+    it without the reference where the restatement has no entry point of that name."""
+    def wrap(fn):
+        @functools.wraps(fn)
+        def method(self, *args, **kw):
+            compute = fn if self._real or stand_in is None else getattr(RefMap, stand_in)
+            return _ask(self._real, self._state, fn.__name__, [args, kw], lambda: compute(self, *args, **kw))
+        return method
+    return wrap
+
+
+def _changes_state(fn):
+    """A RefMap call that changes the map: folded into the history the answers are keyed by."""
+    @functools.wraps(fn)
+    def method(self, *args, **kw):
+        self._state = _digest(self._state, fn.__name__, args, kw)
+        return fn(self, *args, **kw)
+    return method
+
+
 class RefMap(_CpuMap):
+    """The unmodified reference (oracle/_ref/libufo_ref.so).  Where it has not been built, the C
+    restatement stands in for it and every answer is checked against the reference's recorded
+    answer to the same question after the same history (tests/golden/reference/answers.npz)."""
     _path = REF_SO
     _prefix = "ufo_ref_"
 
+    def __init__(self, resolution, depth_levels=16, automatic_pruning=True, color=False, **model):
+        self._real = have_ref()
+        self._tracking, self._changed = False, []   # change detection of the stand-in
+        if not self._real:
+            self._path, self._prefix = ORACLE_SO, "ufo_oracle_"
+        self._kw = dict(automatic_pruning=automatic_pruning, color=color, **model)
+        self._state = _digest("RefMap", float(resolution), int(depth_levels), self._kw)
+        super().__init__(resolution, depth_levels, **self._kw)
+
+    set_value_volume = _changes_state(_CpuMap.set_value_volume)
+    read_data = _changes_state(_asked()(_CpuMap.read_data))
+    walk = _asked()(_CpuMap.walk)
+    node = _asked()(_CpuMap.node)
+    compute_ray = _asked()(_CpuMap.compute_ray)
+    to_key = _asked()(_CpuMap.to_key)
+    to_code = _asked()(_CpuMap.to_code)
+    key_to_code = _asked()(_CpuMap.key_to_code)
+    code_to_key = _asked()(_CpuMap.code_to_key)
+    key_to_coord = _asked()(_CpuMap.key_to_coord)
+    move_line_inside = _asked()(_CpuMap.move_line_inside)
+    change_bbox = _asked()(_CpuMap.change_bbox)
+    sensor_model = _asked()(_CpuMap.sensor_model)
+    write_data = _asked()(_CpuMap.write_data)
+    write = _asked()(_CpuMap.write)
+
+    @_asked()
+    def free_set(self, origin, ends, depth=0, simple=False, early_stopping=0):
+        """The free set, sorted (the reference and the restatement list it in different orders)."""
+        return np.sort(_CpuMap.free_set(self, origin, ends, depth, simple, early_stopping))
+
+    @_asked("_oracle_write_region")
     def write_region(self, box=None, min_depth=0):
         """Octree::write(stream, AABB(min, max) or whole map, False, min_depth): file image."""
         b = None if box is None else np.ascontiguousarray(np.concatenate([box[0], box[1]]), np.float64)
@@ -293,6 +466,16 @@ class RefMap(_CpuMap):
         assert self.api["write_region"](self.h, bp, int(min_depth), buf.ctypes.data, n) == n
         return buf.tobytes()
 
+    def _oracle_header(self, compressed, size):
+        image = _CpuMap.write(self)
+        return image[:image.index(b"compressed ")] + b"compressed %d\nuncompressed_data_size %d\ndata\n" % (
+            compressed, size)
+
+    def _oracle_write_region(self, box=None, min_depth=0):
+        data = _CpuMap.write_data(self, box, min_depth)
+        return self._oracle_header(0, len(data)) + data
+
+    @_asked("_oracle_value_field")
     def value_field(self):
         """Same result as _CpuMap.value_field, produced by the harness in one ordered tree walk
         (no numpy expansion / sort: full-size maps hold ~10^8 voxels)."""
@@ -306,8 +489,12 @@ class RefMap(_CpuMap):
             assert got == n
         return codes, occ, rgb
 
+    def _oracle_value_field(self):
+        return expand_value_field(*_CpuMap.walk(self, True)[:4])
+
+    @_asked("_oracle_leaves")
     def leaves(self, occupied=True, free=True, unknown=False, box=None, min_depth=0):
-        """The reference's beginLeaves(...) iteration: (codes, depths, occ) in iteration order."""
+        """The reference's beginLeaves(...) iteration: (codes, depths, occ), sorted by code."""
         b = None if box is None else np.ascontiguousarray(np.concatenate([box[0], box[1]]), np.float64)
         bp = None if b is None else b.ctypes.data
         n = self.api["leaves"](self.h, int(occupied), int(free), int(unknown), bp, int(min_depth), None, None, None, 0)
@@ -317,8 +504,35 @@ class RefMap(_CpuMap):
         if n:
             self.api["leaves"](self.h, int(occupied), int(free), int(unknown), bp, int(min_depth), codes.ctypes.data,
                                depths.ctypes.data, occ.ctypes.data, n)
-        return codes, depths, occ
+        order = np.argsort(codes, kind="stable")
+        return codes[order], depths[order], occ[order]
 
+    def _oracle_leaves(self, occupied=True, free=True, unknown=False, box=None, min_depth=0):
+        """Leaves at or below min_depth and the nodes at min_depth, filtered by state and box."""
+        lc, ld, lo, _, _ = _CpuMap.walk(self, True)
+        ic, idp, io, _, _ = _CpuMap.walk(self, False)
+        top = idp == min_depth
+        low = ld >= min_depth
+        codes = np.concatenate([lc[low], ic[top]])
+        depths = np.concatenate([ld[low], idp[top]]).astype(np.uint32)
+        occ = np.concatenate([lo[low], io[top]])
+        occ_thr, free_thr = _CpuMap.sensor_model(self)[:2]
+        o64 = occ.astype(np.float64)
+        is_occ, is_free = o64 > occ_thr, o64 < free_thr
+        keep = (occupied & is_occ) | (free & is_free) | (unknown & ~is_occ & ~is_free)
+        if box is not None:
+            key = np.zeros((len(codes), 3), np.float64)
+            for i in range(21):
+                for a in range(3):
+                    key[:, a] += ((codes >> np.uint64(3 * i + a)) & np.uint64(1)).astype(np.float64) * float(1 << i)
+            lo = (key - float(1 << (self.depth_levels - 1))) * self.resolution
+            size = (self.resolution * np.ldexp(1.0, depths.astype(np.int32)))[:, None]
+            keep &= ((lo <= np.asarray(box[1])) & (lo + size >= np.asarray(box[0]))).all(axis=1)
+        codes, depths, occ = codes[keep], depths[keep], occ[keep]
+        order = np.argsort(codes, kind="stable")
+        return codes[order], depths[order], occ[order]
+
+    @_asked("_oracle_write_compressed")
     def write_compressed(self, min_depth=0, acceleration=1, level=0):
         """Octree::write(ostream, compress=True, ...): LZ4-compressed file image (b"" on failure)."""
         n = self.api["write_compressed"](self.h, int(min_depth), int(acceleration), int(level), None, 0)
@@ -327,26 +541,89 @@ class RefMap(_CpuMap):
             assert self.api["write_compressed"](self.h, int(min_depth), int(acceleration), int(level), buf.ctypes.data, n) == n
         return buf[:n].tobytes()
 
+    def _oracle_write_compressed(self, min_depth=0, acceleration=1, level=0):
+        """The node stream through the liblz4 calls the reference makes (octree.h compressData)."""
+        data = _CpuMap.write_data(self, None, min_depth)
+        lz4 = C.CDLL("liblz4.so.1")
+        bound = lz4.LZ4_compressBound(len(data))
+        out = C.create_string_buffer(max(bound, 1))
+        if level <= 0:
+            n = lz4.LZ4_compress_fast(data, out, len(data), bound, int(acceleration))
+        else:
+            n = lz4.LZ4_compress_HC(data, out, len(data), bound, int(level))
+        return self._oracle_header(1, len(data)) + out.raw[:n] if n >= 0 else b""
+
+    @_changes_state
     def enable_change_detection(self, enable=True):
-        self.api["enable_changes"](self.h, int(enable))
+        if self._real:
+            self.api["enable_changes"](self.h, int(enable))
+        else:
+            self._tracking = enable
 
+    @_changes_state
     def reset_change_detection(self):
-        self.api["reset_changes"](self.h)
+        if self._real:
+            self.api["reset_changes"](self.h)
+        else:
+            self._changed = []
 
+    @_changes_state
+    def insert(self, origin, xyz, rgb=None, max_range=-1.0, depth=0, **kw):
+        kw.update(rgb=rgb, max_range=max_range, depth=depth)
+        if self._real or not self._tracking:
+            return _CpuMap.insert(self, origin, xyz, **kw)
+        before = self._oracle_value_field()
+        secs = _CpuMap.insert(self, origin, xyz, **kw)
+        after = self._oracle_value_field()
+        # voxels whose value is not what it was: new ones, and old ones with another value
+        changed = np.ones(len(after[0]), bool)
+        if len(before[0]):
+            i = np.minimum(np.searchsorted(before[0], after[0]), len(before[0]) - 1)
+            changed = (before[0][i] != after[0]) | (before[1][i].view(np.uint32) != after[1].view(np.uint32))
+        changed = after[0][changed]
+        if depth:
+            # the reference records the hit voxels at depth 0 and the free space as the depth-d
+            # nodes it updated (a depth-d code has its 3 d low bits set)
+            pts = _f64(xyz).reshape(-1, 3)
+            if max_range >= 0:
+                pts = pts[np.linalg.norm(pts - _f64(origin), axis=1) <= max_range]
+            hits = np.unique(np.array([_CpuMap.to_code(self, q, 0) for q in pts], np.uint64))
+            low = np.uint64((1 << (3 * depth)) - 1)
+            free = np.unique((np.setdiff1d(changed, hits) & ~low) | low)
+            self._changed.append((np.intersect1d(changed, hits), 0))
+            self._changed.append((free, depth))
+        else:
+            self._changed.append((changed, 0))
+        return secs
+
+    @_asked("_oracle_changed_codes")
     def changed_codes(self):
-        """(sorted codes, depths) of the reference's changes_ set."""
+        """(codes, depths) of the reference's changes_ set, sorted by code, then depth."""
         n = self.api["changes"](self.h, None, None, 0)
         codes = np.empty(n, np.uint64)
         depths = np.empty(n, np.uint32)
         if n:
             self.api["changes"](self.h, codes.ctypes.data, depths.ctypes.data, n)
-        order = np.argsort(codes, kind="stable")
+        order = np.lexsort((depths, codes))
         return codes[order], depths[order]
 
+    def _oracle_changed_codes(self):
+        codes = np.concatenate([c for c, _ in self._changed] + [np.empty(0, np.uint64)])
+        depths = np.concatenate([np.full(len(c), d, np.uint32) for c, d in self._changed] + [np.empty(0, np.uint32)])
+        both = np.unique(np.stack([codes, depths.astype(np.uint64)], axis=1), axis=0)
+        return both[:, 0].copy(), both[:, 1].astype(np.uint32)
+
+    @_asked("_oracle_field_count")
     def field_count(self):
         """Number of non-default depth-0 voxels (collapsed nodes counted as 8^depth)."""
         return int(self.api["field"](self.h, None, None, None, 0))
 
+    def _oracle_field_count(self):
+        _, depths, occ, rgb, _ = _CpuMap.walk(self, True)
+        keep = (occ != 0) | rgb.any(axis=1)
+        return int((np.uint64(1) << (np.uint64(3) * depths[keep].astype(np.uint64))).sum())
+
+    @_asked("_oracle_node_batch")
     def node_batch(self, codes, depths=0):
         """Deepest existing node on the path to each code: (occ f32, rgb u8[n,3], flags, depth found)."""
         codes = np.ascontiguousarray(codes, dtype=np.uint64)
@@ -360,14 +637,38 @@ class RefMap(_CpuMap):
                                rgb.ctypes.data, flags.ctypes.data, fd.ctypes.data)
         return occ, rgb, flags, fd
 
+    def _oracle_node_batch(self, codes, depths=0):
+        codes = np.ascontiguousarray(codes, dtype=np.uint64)
+        depths = np.broadcast_to(depths, codes.shape)
+        occ = np.empty(len(codes), np.float32)
+        rgb = np.zeros((len(codes), 3), np.uint8)
+        flags = np.empty(len(codes), np.uint8)
+        fd = np.empty(len(codes), np.uint32)
+        for i in range(len(codes)):
+            _, occ[i], rgb[i], flags[i], fd[i] = _CpuMap.node(self, codes[i], depths[i])
+        return occ, rgb, flags, fd
+
+    @_changes_state
     def clear(self, resolution, depth_levels):
         """Octree::clear(resolution, depth_levels)."""
-        self.api["clear"](self.h, float(resolution), int(depth_levels))
+        if self._real:
+            self.api["clear"](self.h, float(resolution), int(depth_levels))
+        else:
+            self.close()
+            _CpuMap.__init__(self, resolution, depth_levels, **self._kw)
 
+    @_changes_state
+    @_asked("_oracle_read")
     def read(self, image):
         """Octree::read(istream): replace the map's content by a file image."""
         buf = np.frombuffer(image, np.uint8)
         return bool(self.api["read"](self.h, buf.ctypes.data, len(buf)))
+
+    def _oracle_read(self, image):
+        """The node stream behind the header into an emptied map of the same geometry."""
+        self.close()
+        _CpuMap.__init__(self, self.resolution, self.depth_levels, **self._kw)
+        return _CpuMap.read_data(self, image[image.index(b"data\n") + 5:])
 
 
 class OracleMap(_CpuMap):

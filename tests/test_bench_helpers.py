@@ -58,3 +58,46 @@ def test_configs_match_baseline_json():
     assert b.CONFIGS[3]["resolution"] == 0.002 and b.CONFIGS[3]["color"]
     assert b.CONFIGS[4]["resolution"] == 0.05 and b.CONFIGS[4]["max_range"] == 100.0
     assert "points" in json.dumps(base).lower()
+
+
+def test_dump_outputs_writes_the_field_and_counters(tmp_path):
+    """--dump-outputs: keys decoded from the voxel codes, float dtypes, a sample of a field above the
+    cap that does not depend on the order the device emitted the voxels in."""
+    import numpy as np
+    b = _bench()
+    rng = np.random.default_rng(0)
+    keys = rng.integers(0, 1 << 16, (3000, 3)).astype(np.uint64)
+    codes = np.zeros(len(keys), np.uint64)
+    for i in range(16):
+        for a in range(3):
+            codes |= ((keys[:, a] >> np.uint64(i)) & np.uint64(1)) << np.uint64(3 * i + a)
+    codes, idx = np.unique(codes, return_index=True)
+    keys = keys[idx]
+
+    class FakeMap:
+        def __init__(self, perm):
+            self.perm = perm
+
+        def wait(self):
+            pass
+
+        def value_field(self, sort=True):
+            occ = (codes % np.uint64(97)).astype(np.float32)
+            rgb = np.stack([(codes % np.uint64(251)).astype(np.uint8)] * 3, axis=1)
+            return codes[self.perm], occ[self.perm], rgb[self.perm]
+
+        def stats(self):
+            return {k: i for i, k in enumerate(b.COUNTER_NAMES)}
+
+    b.dump_outputs(str(tmp_path / "all"), FakeMap(np.arange(len(codes))), True)
+    k = np.load(tmp_path / "all" / "voxel_keys.npy")
+    assert k.dtype == np.float64 and np.array_equal(k, keys.astype(np.float64))
+    assert np.load(tmp_path / "all" / "log_odds.npy").dtype == np.float32
+    assert np.load(tmp_path / "all" / "rgb.npy").dtype == np.float32
+    assert list(np.load(tmp_path / "all" / "scan_counters.npy")) == list(range(len(b.COUNTER_NAMES)))
+    b.DUMP_MAX_VOXELS = 500
+    for name in ("a", "b"):
+        b.dump_outputs(str(tmp_path / name), FakeMap(rng.permutation(len(codes))), False)
+    a_, b_ = (np.load(tmp_path / n / "voxel_keys.npy") for n in ("a", "b"))
+    assert 300 < len(a_) < 700 and np.array_equal(a_, b_)
+    assert not (tmp_path / "a" / "rgb.npy").exists()

@@ -5,7 +5,7 @@ reference's own Octree::read."""
 import numpy as np
 import pytest
 
-from oracle_lib import OracleMap, RefMap, have_ref
+from oracle_lib import OracleMap, RefMap
 from ufomap_b200 import scans
 from ufomap_b200.capi import Map
 
@@ -13,10 +13,7 @@ pytestmark = pytest.mark.gpu
 
 
 def _cpu_maps(color, **kw):
-    maps = [OracleMap(color=color, **kw)]
-    if have_ref():
-        maps.append(RefMap(color=color, **kw))
-    return maps
+    return [OracleMap(color=color, **kw), RefMap(color=color, **kw)]
 
 
 def _scenario(name):
@@ -60,7 +57,6 @@ def test_image_is_byte_identical(name, pruning, tmp_path):
     gpu.close()
 
 
-@pytest.mark.skipif(not have_ref(), reason="reference harness not built")
 @pytest.mark.parametrize("name,depth", [("velodyne", 0), ("rgbd_color_discrete", 0), ("velodyne", 2)])
 @pytest.mark.parametrize("expanded", [False, True])
 def test_image_reads_back_in_the_reference(name, depth, expanded):
@@ -114,7 +110,6 @@ def test_partial_and_truncated_stream(name):
     gpu.close()
 
 
-@pytest.mark.skipif(not have_ref(), reason="reference harness not built")
 def test_region_file_and_reset(tmp_path):
     """save_map (Octree::write(filename, bounding volume, compress, depth), server.cpp:381-392) and
     reset (Octree::clear(resolution, depth_levels), server.cpp:364-378)."""
@@ -151,8 +146,6 @@ def test_compressed_image_matches_the_reference(name):
     """write(compress=True): one LZ4 block behind the header (octree.h:1428-1456).  The same liblz4
     on both sides -> byte-identical to the reference's own compressed file, for the fast and the
     HC compressor; the data-only form decompresses to the uncompressed node stream."""
-    if not have_ref():
-        pytest.skip("needs the compiled reference")
     import ctypes
     kw, inserts, color = _scenario(name)
     gpu, ref = Map(color=color, initial_blocks=1 << 12, **kw), RefMap(color=color, **kw)

@@ -2,15 +2,15 @@
 seeded inputs.  Log-odds are compared bit-for-bit, codes/keys exactly, colours +-1.
 
 The oracle is oracle/libufo_oracle.so (plain-C restatement, pinned to the real
-reference by tests/test_oracle_vs_reference.py and tests/golden/); when the
-prebuilt reference harness travelled (oracle/_ref/libufo_ref.so) the same cases
-are also checked directly against it.
+reference by tests/test_oracle_vs_reference.py and tests/golden/); the same cases
+are also checked against the reference itself (oracle/_ref/libufo_ref.so, or its
+recorded answers where it is not built: tests/oracle_lib.py RefMap).
 """
 import numpy as np
 import pytest
 
 from helpers import assert_value_fields_equal, check_inner_against_field
-from oracle_lib import OracleMap, RefMap, have_ref
+from oracle_lib import OracleMap, RefMap
 from ufomap_b200 import scans
 from ufomap_b200.capi import Map, UfoError, E_UNSUPPORTED
 
@@ -20,7 +20,7 @@ pytestmark = pytest.mark.gpu
 def _run_case(map_kw, inserts, color=False, color_tol=1, with_ref=True, levels=(1, 2, 3, 4, 5, 6, 9, 16)):
     gpu = Map(color=color, initial_blocks=1 << 14, **map_kw)
     cpus = [OracleMap(color=color, **map_kw)]
-    if with_ref and have_ref():
+    if with_ref:
         cpus.append(RefMap(color=color, **map_kw))
     for ins in inserts:
         gpu.insert(**ins)
@@ -370,7 +370,7 @@ def test_set_value_volume(color):
     next scans on top must match the reference."""
     kw = dict(resolution=0.05)
     gpu = Map(color=color, initial_blocks=1 << 12, **kw)
-    cpus = [OracleMap(color=color, **kw)] + ([RefMap(color=color, **kw)] if have_ref() else [])
+    cpus = [OracleMap(color=color, **kw), RefMap(color=color, **kw)]
     rng = np.random.default_rng(23)
     res = kw["resolution"]
     depths = [0, 0, 0, 0] if color else [0, 1, 2, 3, 4, 0]
@@ -408,8 +408,6 @@ def test_set_value_volume(color):
 def test_change_detection_matches_the_reference_set():
     """enableChangeDetection / changes (occupancy_map_base.h:779-790): the set of nodes whose value
     changed since the last reset, against the reference's own changes_ set."""
-    if not have_ref():
-        pytest.skip("needs the compiled reference")
     gpu, ref = Map(0.1), RefMap(0.1)
     gpu.enable_change_detection(True)
     ref.enable_change_detection(True)
@@ -475,8 +473,6 @@ def test_filtered_leaf_iteration_matches_the_reference():
     """beginLeaves(occupied, free, unknown, contains=false, min_depth) [+ AABB]
     (occupancy_map_base.h:130-216) against ufo_b200_export_nodes: same set of depth-d cells with
     the same values (a leaf the reference keeps collapsed above d is expanded into its cells)."""
-    if not have_ref():
-        pytest.skip("needs the compiled reference")
     gpu, ref = Map(0.1), RefMap(0.1)
     for k in range(3):
         o, p = scans.velodyne64(k=k, rings=16, azimuths=256)

@@ -1,7 +1,7 @@
 """GPU parity at the BASELINE configs' REAL sizes against the compiled, unmodified reference
-(oracle/_ref/libufo_ref.so; falls back to the C restatement when the prebuilt harness did not
-travel).  The whole value field is compared bit for bit (log-odds) / +-1 (colour), inner
-aggregates on random samples of every level, and the change box.
+(oracle/_ref/libufo_ref.so; where it is not built, the C restatement checked against the
+reference's recorded answers: tests/oracle_lib.py RefMap).  The whole value field is compared bit
+for bit (log-odds) / +-1 (colour), inner aggregates on random samples of every level, and the change box.
 
 The reference needs minutes per case on one core (BASELINE.md section 4: ~1 k points/s), so
 all cases are integrated on the CPU concurrently in background threads (the harness calls
@@ -21,7 +21,7 @@ import numpy as np
 import pytest
 
 from helpers import assert_value_fields_equal, check_inner_sampled, sorted_field_large
-from oracle_lib import OracleMap, RefMap, have_ref
+from oracle_lib import RefMap
 from ufomap_b200 import scans
 from ufomap_b200.capi import Map
 
@@ -60,18 +60,17 @@ def _cases():
 
 
 def _cpu_run(case):
-    cls = RefMap if have_ref() else OracleMap
-    m = cls(color=case["color"], **case["map_kw"])
+    m = RefMap(color=case["color"], **case["map_kw"])
     secs = 0.0
     for ins in case["inserts"]:
         secs += m.insert(**ins)
     bbox = m.change_bbox()
     model = m.sensor_model()
     if case.get("sampled"):
-        return dict(map=m, bbox=bbox, model=model, secs=secs, kind=cls.__name__)
+        return dict(map=m, bbox=bbox, model=model, secs=secs, kind="RefMap")
     field = m.value_field()
     m.close()
-    return dict(field=field, bbox=bbox, model=model, secs=secs, kind=cls.__name__)
+    return dict(field=field, bbox=bbox, model=model, secs=secs, kind="RefMap")
 
 
 @pytest.fixture(scope="module")
@@ -126,8 +125,6 @@ def test_config3_full_size_coarse_insert_color(cpu_results, name):
     """Full-size #3 at insert depth 4 / 6: number of non-default voxels, and occupancy (bit-exact) +
     colour (+-1) of 2 M voxels sampled along the rays (free space) and at the end points (hits)."""
     cases, futures = cpu_results
-    if not have_ref():
-        pytest.skip("needs the compiled reference (batched node lookup)")
     case = cases[name]
     gpu = Map(color=True, initial_bricks=1 << 19, **case["map_kw"])
     rng = np.random.default_rng(3)

@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 
 from helpers import assert_value_fields_equal
-from oracle_lib import OracleMap, RefMap, have_ref
+from oracle_lib import OracleMap, RefMap
 from ufomap_b200 import capi, scans
 from ufomap_b200.capi import Map
 
@@ -72,7 +72,7 @@ def test_sensors_merged_in_sensor_order():
     res, world = 0.04, 2
     maps = _ranks(world, res, bricks=1 << 16)
     single = Map(res, initial_bricks=1 << 16)
-    cpus = [OracleMap(res)] + ([RefMap(res)] if have_ref() else [])
+    cpus = [OracleMap(res), RefMap(res)]
     for k in range(2):
         keep = []
         for s, m in enumerate(maps):
