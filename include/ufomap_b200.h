@@ -266,7 +266,10 @@ int ufo_b200_reset_change_bbox(ufo_b200_map* m);
  * since the last reset (updateOccupancy returned true, :1070, :1094, :1106).  Recorded per voxel on
  * the device; ufo_b200_changed_codes returns the set at `depth` -- the insert depth the caller
  * used, 0 for the server's default -- as Code values (with the centre bits a Code built from a
- * depth-d Key carries), unordered like the reference's CodeSet.  codes == NULL: count only. */
+ * depth-d Key carries), unordered like the reference's CodeSet.  codes == NULL: count only.
+ * enable == 0 pauses the recording and keeps the set, as the reference does: it grows with the map,
+ * ufo_b200_changed_codes / ufo_b200_reset_change_detection / ufo_b200_clear act on it as they do
+ * while recording, and enabling again resumes recording into it. */
 int ufo_b200_enable_change_detection(ufo_b200_map* m, int enable);
 int ufo_b200_reset_change_detection(ufo_b200_map* m);
 int ufo_b200_changed_codes(ufo_b200_map* m, uint32_t depth, uint64_t* codes, size_t cap, size_t* n);

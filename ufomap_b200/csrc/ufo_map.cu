@@ -57,30 +57,80 @@ struct CudaError {
 		if (e__ != cudaSuccess) throw CudaError{e__, #call, __LINE__}; \
 	} while (0)
 
-template <class T>
-void dev_alloc(T*& p, size_t n, int fill_byte, cudaStream_t s, size_t& total)
-{
-	p = nullptr;
-	if (n == 0) n = 1;
-	CK(cudaMalloc(reinterpret_cast<void**>(&p), n * sizeof(T)));
-	CK(cudaMemsetAsync(p, fill_byte, n * sizeof(T), s));
-	total += n * sizeof(T);
-}
+enum class Mem { kDevice, kPinned };
 
-// grow p from old_n to new_n elements (new part filled with fill_byte)
-template <class T>
-void dev_grow(T*& p, size_t old_n, size_t new_n, int fill_byte, cudaStream_t s, size_t& total)
+// Owns one allocation of T: device memory, or pinned host memory.  A buffer made with a byte
+// count adds its size to it while it holds memory, so that the count is always the sum over the
+// owner's live buffers (ufo_b200_scan_stats::device_bytes).
+template <class T, Mem kMem = Mem::kDevice>
+class Buffer
 {
-	if (!p) return;
-	T* q = nullptr;
-	CK(cudaMalloc(reinterpret_cast<void**>(&q), new_n * sizeof(T)));
-	CK(cudaMemcpyAsync(q, p, old_n * sizeof(T), cudaMemcpyDeviceToDevice, s));
-	CK(cudaMemsetAsync(q + old_n, fill_byte, (new_n - old_n) * sizeof(T), s));
-	CK(cudaStreamSynchronize(s));
-	CK(cudaFree(p));
-	p = q;
-	total += (new_n - old_n) * sizeof(T);
-}
+public:
+	Buffer(size_t* total = nullptr) : total_(total) {}
+	Buffer(Buffer&& o) noexcept : p_(o.p_), n_(o.n_), total_(o.total_)
+	{
+		o.p_ = nullptr;
+		o.n_ = 0;
+	}
+	Buffer& operator=(Buffer&& o) noexcept
+	{
+		std::swap(p_, o.p_);
+		std::swap(n_, o.n_);
+		std::swap(total_, o.total_);
+		return *this;
+	}
+	~Buffer() { reset(); }
+
+	T* get() const { return p_; }
+	T* operator->() const { return p_; }
+	T& operator*() const { return *p_; }
+	size_t size() const { return n_; }
+	size_t bytes() const { return n_ * sizeof(T); }
+
+	void reset()
+	{
+		if (!p_) return;
+		if (kMem == Mem::kPinned) cudaFreeHost(p_);
+		else cudaFree(p_);
+		if (total_) *total_ -= bytes();
+		p_ = nullptr;
+		n_ = 0;
+	}
+
+	// n elements (at least one); the contents are not kept.  fill >= 0: every byte is set to it on s.
+	void resize(size_t n, int fill = -1, cudaStream_t s = nullptr)
+	{
+		reset();
+		n = std::max<size_t>(n, 1);
+		if (kMem == Mem::kPinned) CK(cudaHostAlloc(reinterpret_cast<void**>(&p_), n * sizeof(T), cudaHostAllocDefault));
+		else CK(cudaMalloc(reinterpret_cast<void**>(&p_), n * sizeof(T)));
+		n_ = n;
+		if (total_) *total_ += bytes();
+		if (fill >= 0) CK(cudaMemsetAsync(p_, fill, bytes(), s));
+	}
+
+	// n elements, the contents kept and the new part set to fill; waits for s
+	void grow(size_t n, int fill, cudaStream_t s)
+	{
+		Buffer q(total_);
+		q.resize(n);
+		CK(cudaMemcpyAsync(q.p_, p_, bytes(), cudaMemcpyDeviceToDevice, s));
+		CK(cudaMemsetAsync(q.p_ + n_, fill, q.bytes() - bytes(), s));
+		CK(cudaStreamSynchronize(s));
+		*this = std::move(q);
+	}
+
+	// sets the first n elements (all of them by default) to `byte` on s
+	void fill(int byte, cudaStream_t s, size_t n = ~size_t(0)) const
+	{
+		CK(cudaMemsetAsync(p_, byte, std::min(n, n_) * sizeof(T), s));
+	}
+
+private:
+	T* p_ = nullptr;
+	size_t n_ = 0;
+	size_t* total_;
+};
 
 double to_logit(double p) { return std::log(p / (1.0 - p)); }
 }  // namespace
@@ -109,33 +159,40 @@ struct ufo_b200_map {
 	cudaEvent_t ev_copy0 = nullptr, ev_copied = nullptr;
 	// sensor model as the reference stores it (double log-odds)
 	double occ_thr_log = 0, free_thr_log = 0, hit_log = 0, miss_log = 0, cmin_log = 0, cmax_log = 0;
-	// host mirror of the counters (pinned)
-	Counters* h_ctr = nullptr;
+	// Every allocation of the map is one of the buffers below; device_bytes is the sum of the sizes
+	// of the device buffers (each adds and removes its own).
+	size_t device_bytes = 0;
+	// brick and upper-node pools: one buffer per array of for_each_pool_array, which also points
+	// the DeviceMap fields (and the views below) at them
+	std::vector<Buffer<unsigned char>> pool;
+	uint32_t* d_list[2] = {nullptr, nullptr};  // dirty lists of the upper-level pass
+	unsigned long long* chg_mask = nullptr;    // change mask (DeviceMap::chg_mask while recording)
+	bool chg_recording = false;
+	Buffer<ulonglong2> bh_tab{&device_bytes};
+	Buffer<unsigned long long> uh_keys{&device_bytes};
+	Buffer<uint32_t> uh_vals{&device_bytes};
+	Buffer<Counters> ctr{&device_bytes};
+	Buffer<Counters, Mem::kPinned> h_ctr;  // host mirror of the counters
 	// scan staging: two point buffers, so that the H2D copy of scan k+1 overlaps scan k
-	void* d_points[2] = {nullptr, nullptr};
-	size_t d_points_cap[2] = {0, 0};
+	Buffer<unsigned char> d_points[2] = {&device_bytes, &device_bytes};
 	uint32_t stage = 0;
-	double* d_ray_end = nullptr;
-	uint32_t* d_hit_tab = nullptr;
-	size_t ray_cap = 0;
-	unsigned long long* d_tab_keys = nullptr;
-	uint32_t* d_tab_min = nullptr;
-	uint32_t tab_size = 0;
-	uint32_t* d_list[2] = {nullptr, nullptr};
+	Buffer<double> d_ray_end{&device_bytes};  // [ray capacity][3]
+	Buffer<uint32_t> d_hit_tab{&device_bytes};  // [ray capacity]
+	Buffer<unsigned long long> d_tab_keys{&device_bytes};
+	Buffer<uint32_t> d_tab_min{&device_bytes};
 	// generic marking path: ray-walk records
-	QEntry* d_seg = nullptr;
-	unsigned long long seg_cap = 0;
-	uint32_t *d_seg_base = nullptr, *d_seg_count = nullptr;
-	uint32_t* d_order = nullptr;
-	unsigned long long* d_nodes = nullptr;  // insert depth 5/6: free-space nodes of the scan
+	Buffer<QEntry> d_seg{&device_bytes};
+	Buffer<uint32_t> d_seg_base{&device_bytes}, d_seg_count{&device_bytes}, d_order{&device_bytes};
+	Buffer<unsigned long long> d_nodes{&device_bytes};  // insert depth 5/6: free-space nodes of the scan
 	// fused walk: segments, validity masks, per-ray constants
-	Item* d_items = nullptr;
-	uint32_t* d_vmask = nullptr;
-	RayConst* d_rc = nullptr;
-	size_t item_cap = 0;
+	Buffer<Item> d_items{&device_bytes};
+	Buffer<uint32_t> d_vmask{&device_bytes};
+	Buffer<RayConst> d_rc{&device_bytes};
+	// dense scan volume
+	Buffer<unsigned long long> vol{&device_bytes}, vol_dirty{&device_bytes};
+	Buffer<uint32_t> vol_list{&device_bytes};
 	// bookkeeping
 	uint32_t n_blocks = 0, n_bricks = 0, n_upper = 0;  // host view after the last completed scan
-	size_t device_bytes = 0;
 	int profiling = 0;
 	int force_records = 0;  // UFO_B200_MARK=records: always use the record path (A/B runs)
 	int k3_blocks = 0;      // UFO_B200_K3_BLOCKS: resident K3 CTAs per SM (0: the kernel's launch bound)
@@ -149,19 +206,30 @@ struct ufo_b200_map {
 	bool stats_pending = false;
 	PendingScan pending;
 	bool poisoned = false;
-	unsigned long long* chg_paused = nullptr;  // change masks kept while detection is switched off
 	// routed multi-GPU mode
-	unsigned char* route_inbox = nullptr;  // this rank's inbox: [2 parities][world sources] regions
+	Buffer<unsigned char> route_inbox{&device_bytes};  // this rank's inbox: [2 parities][world sources] regions
+	Buffer<RouteTable> route{&device_bytes};
 	size_t route_region = 0, route_miss_off = 0, route_hit_off = 0;
 	void* route_peer[kMaxRanks] = {};
-	RouteTable* h_route = nullptr;  // pinned mirror, pushed before every mark pass
-	uint32_t* h_route_flag = nullptr;
+	Buffer<RouteTable, Mem::kPinned> h_route;  // pinned mirror, pushed before every mark pass
+	Buffer<uint32_t, Mem::kPinned> h_route_flag;
 	uint32_t route_parity = 0, route_cap_m = 0, route_cap_h = 0;
 	int route_stage = 0;  // 0 idle, 1 marked (waiting for the apply calls), 2 applied
 	double min_change[3], max_change[3];
 	std::string err;
 	int sm_count = 148;
 	int ray_blocks_per_sm = 4, walk_blocks_per_sm = 4;
+
+	// the buffers free themselves after this; the caller has waited for the stream
+	~ufo_b200_map()
+	{
+		for (cudaEvent_t e : ev)
+			if (e) cudaEventDestroy(e);
+		if (ev_copy0) cudaEventDestroy(ev_copy0);
+		if (ev_copied) cudaEventDestroy(ev_copied);
+		if (own_stream) cudaStreamDestroy(own_stream);
+		if (copy_stream) cudaStreamDestroy(copy_stream);
+	}
 
 	void set_error(const char* fmt, ...)
 	{
@@ -211,64 +279,123 @@ void reset_bbox(Map* m)
 	}
 }
 
+// ---- brick and upper-node pools --------------------------------------------------------------
+enum class Unit { kSlot, kBrick, kUpper };  // block slot (64 per brick), brick, upper node
+// when an array exists: always, on colour maps, or from the first out-of-tree key (alias masks) /
+// the first enableChangeDetection (change mask) on
+enum class Exists { kAlways, kColour, kAlias, kChange };
+
+struct PoolArray {
+	Buffer<unsigned char>& buf;  // empty while the array does not exist
+	Unit unit;
+	size_t unit_bytes;  // bytes per unit
+	int fill;           // byte the array (and every part added by a growth) starts as
+	Exists exists;
+	bool cleared;  // ufo_b200_clear resets the part in use
+};
+
+size_t capacity(const DeviceMap& M, Unit u)
+{
+	return u == Unit::kSlot ? (size_t)M.brick_cap * 64 : (u == Unit::kBrick ? M.brick_cap : M.up_cap);
+}
+
+size_t in_use(const Map* m, Unit u)
+{
+	return u == Unit::kSlot ? (size_t)m->n_bricks * 64 : (u == Unit::kBrick ? m->n_bricks : m->n_upper);
+}
+
+// Calls f(PoolArray) for every array of the two pools, then points the array's view (a DeviceMap
+// field or a field of the map) at its buffer.  The hash tables and counters are sized on their own.
+template <class F>
+void for_each_pool_array(Map* m, F&& f)
+{
+	DeviceMap& M = m->M;
+	size_t i = 0;
+	auto array = [&](auto*& view, Unit unit, size_t per_unit, int fill, Exists exists, bool cleared) {
+		using T = std::remove_reference_t<decltype(*view)>;
+		if (i == m->pool.size()) m->pool.emplace_back(&m->device_bytes);
+		Buffer<unsigned char>& buf = m->pool[i++];
+		f(PoolArray{buf, unit, per_unit * sizeof(T), fill, exists, cleared});
+		view = reinterpret_cast<T*>(buf.get());
+	};
+	const Unit S = Unit::kSlot, B = Unit::kBrick, U = Unit::kUpper;
+	const Exists all = Exists::kAlways, colour = Exists::kColour;
+	//    view              unit  per unit  fill  exists          cleared
+	array(M.brick_key,      B,    1,        0,    all,            false);
+	array(M.brick_stamp,    B,    1,        0,    all,            true);
+	array(M.touched,        B,    1,        0,    all,            false);
+	array(M.touched_alt,    B,    1,        0,    all,            false);
+	array(M.touched_mi,     B,    1,        0,    all,            false);
+	array(M.touched_alt_mi, B,    1,        0,    all,            false);
+	array(M.brick_sum3,     B,    8,        0,    all,            false);
+	array(M.brick_sum4,     B,    1,        0,    all,            false);
+	array(M.brick_parent,   B,    1,        0xff, all,            true);
+	array(M.brick_rgb3,     B,    8,        0,    colour,         false);
+	array(M.brick_rgb4,     B,    1,        0,    colour,         false);
+	array(M.leaf,           S,    64,       0,    all,            true);
+	array(M.miss_mask,      S,    1,        0,    all,            true);
+	array(M.hit_mask,       S,    1,        0,    all,            true);
+	array(M.agg2,           S,    1,        0,    all,            true);
+	array(M.meta,           S,    1,        0,    all,            true);
+	array(M.sum1,           S,    8,        0,    all,            false);
+	array(M.leaf_rgb,       S,    64,       0,    colour,         true);
+	array(M.sum1_rgb,       S,    8,        0,    colour,         false);
+	array(M.rgb2,           S,    1,        0,    colour,         false);
+	array(M.alias_miss,     S,    1,        0,    Exists::kAlias, true);
+	array(M.alias_hit,      S,    1,        0,    Exists::kAlias, true);
+	array(m->chg_mask,      S,    1,        0,    Exists::kChange, true);
+	array(M.up_key,         U,    1,        0,    all,            false);
+	array(M.up_agg,         U,    1,        0,    all,            false);
+	array(M.up_stamp,       U,    1,        0,    all,            true);
+	array(M.up_child,       U,    8,        0,    all,            false);
+	array(M.up_valid,       U,    1,        0,    all,            true);
+	array(M.up_parent,      U,    1,        0xff, all,            true);
+	array(M.up_rgb,         U,    1,        0,    colour,         false);
+	array(M.up_child_rgb,   U,    8,        0,    colour,         false);
+	array(m->d_list[0],     U,    1,        0,    all,            false);
+	array(m->d_list[1],     U,    1,        0,    all,            false);
+	// the kernels record changes while chg_mask is set
+	M.chg_mask = m->chg_recording ? m->chg_mask : nullptr;
+}
+
+// allocates the arrays of one kind that do not exist yet, at the pools' capacities
+void alloc_arrays(Map* m, Exists kind)
+{
+	for_each_pool_array(m, [&](const PoolArray& a) {
+		if (a.exists == kind && !a.buf.get()) a.buf.resize(capacity(m->M, a.unit) * a.unit_bytes, a.fill, m->stream);
+	});
+}
+
+// the hash tables: open addressing at a load of at most 1/2, contents not kept
+void alloc_brick_hash(Map* m)
+{
+	DeviceMap& M = m->M;
+	M.bh_mask = std::max(kMinHash, next_pow2(2ull * M.brick_cap)) - 1;
+	m->bh_tab.resize((size_t)M.bh_mask + 1, 0xff, m->stream);
+	M.bh_tab = m->bh_tab.get();
+}
+
+void alloc_upper_hash(Map* m)
+{
+	DeviceMap& M = m->M;
+	M.uh_mask = std::max(kMinHash, next_pow2(2ull * M.up_cap)) - 1;
+	m->uh_keys.resize((size_t)M.uh_mask + 1, 0xff, m->stream);
+	m->uh_vals.resize((size_t)M.uh_mask + 1, 0xff, m->stream);
+	M.uh_keys = m->uh_keys.get();
+	M.uh_vals = m->uh_vals.get();
+}
+
 void alloc_pools(Map* m, uint32_t brick_cap, uint32_t up_cap)
 {
 	DeviceMap& M = m->M;
-	cudaStream_t s = m->stream;
-	size_t& tot = m->device_bytes;
-	const size_t nb = (size_t)brick_cap * 64;  // block slots: 64 consecutive per brick
 	M.brick_cap = brick_cap;
 	M.up_cap = up_cap;
-	M.bh_mask = std::max(kMinHash, next_pow2(2ull * brick_cap)) - 1;
-	M.uh_mask = std::max(kMinHash, next_pow2(2ull * up_cap)) - 1;
-	dev_alloc(M.bh_tab, (size_t)M.bh_mask + 1, 0xff, s, tot);
-	dev_alloc(M.brick_key, brick_cap, 0, s, tot);
-	dev_alloc(M.brick_stamp, brick_cap, 0, s, tot);
-	dev_alloc(M.touched, brick_cap, 0, s, tot);
-	dev_alloc(M.touched_alt, brick_cap, 0, s, tot);
-	dev_alloc(M.touched_mi, brick_cap, 0, s, tot);
-	dev_alloc(M.touched_alt_mi, brick_cap, 0, s, tot);
-	dev_alloc(M.brick_sum3, (size_t)brick_cap * 8, 0, s, tot);
-	dev_alloc(M.brick_sum4, brick_cap, 0, s, tot);
-	dev_alloc(M.leaf, nb * 64, 0, s, tot);
-	dev_alloc(M.miss_mask, nb, 0, s, tot);
-	dev_alloc(M.hit_mask, nb, 0, s, tot);
-	dev_alloc(M.agg2, nb, 0, s, tot);
-	dev_alloc(M.meta, nb, 0, s, tot);
-	dev_alloc(M.sum1, nb * 8, 0, s, tot);
-	dev_alloc(M.uh_keys, (size_t)M.uh_mask + 1, 0xff, s, tot);
-	dev_alloc(M.uh_vals, (size_t)M.uh_mask + 1, 0xff, s, tot);
-	dev_alloc(M.up_key, up_cap, 0, s, tot);
-	dev_alloc(M.up_agg, up_cap, 0, s, tot);
-	dev_alloc(M.up_stamp, up_cap, 0, s, tot);
-	dev_alloc(M.up_child, (size_t)up_cap * 8, 0, s, tot);
-	dev_alloc(M.up_valid, up_cap, 0, s, tot);
-	dev_alloc(M.up_parent, up_cap, 0xff, s, tot);
-	dev_alloc(M.brick_parent, brick_cap, 0xff, s, tot);
-	dev_alloc(m->d_list[0], up_cap, 0, s, tot);
-	dev_alloc(m->d_list[1], up_cap, 0, s, tot);
-	if (M.color) {
-		dev_alloc(M.brick_rgb3, (size_t)brick_cap * 8, 0, s, tot);
-		dev_alloc(M.brick_rgb4, brick_cap, 0, s, tot);
-		dev_alloc(M.leaf_rgb, nb * 64, 0, s, tot);
-		dev_alloc(M.sum1_rgb, nb * 8, 0, s, tot);
-		dev_alloc(M.rgb2, nb, 0, s, tot);
-		dev_alloc(M.up_rgb, up_cap, 0, s, tot);
-		dev_alloc(M.up_child_rgb, (size_t)up_cap * 8, 0, s, tot);
-	}
-	dev_alloc(M.ctr, 1, 0, s, tot);
-}
-
-void free_pools(Map* m)
-{
-	DeviceMap& M = m->M;
-	void* ptrs[] = {M.bh_tab, M.brick_key, M.brick_stamp, M.touched, M.touched_alt, M.touched_mi, M.touched_alt_mi, M.chg_mask, M.vol, M.vol_dirty, M.vol_list, M.route, m->route_inbox, M.brick_sum3, M.brick_sum4, M.brick_rgb3, M.brick_rgb4,
-	                M.leaf, M.leaf_rgb, M.miss_mask, M.hit_mask, M.agg2, M.meta, M.sum1, M.rgb2, M.sum1_rgb,
-	                M.alias_miss, M.alias_hit, M.uh_keys, M.uh_vals, M.up_key, M.up_agg, M.up_rgb, M.up_stamp, M.up_child, M.up_child_rgb, M.up_valid, M.up_parent, M.brick_parent, M.ctr, m->d_list[0],
-	                m->d_list[1], m->d_points[0], m->d_points[1], m->d_ray_end, m->d_hit_tab, m->d_tab_keys, m->d_tab_min,
-	                m->d_seg, m->d_seg_base, m->d_seg_count, m->d_order, m->d_nodes, m->d_items, m->d_vmask, m->d_rc};
-	for (void* p : ptrs)
-		if (p) cudaFree(p);
+	alloc_brick_hash(m);
+	alloc_upper_hash(m);
+	alloc_arrays(m, Exists::kAlways);
+	if (M.color) alloc_arrays(m, Exists::kColour);
+	m->ctr.resize(1, 0, m->stream);
+	M.ctr = m->ctr.get();
 }
 
 void push_counters(Map* m)
@@ -283,7 +410,17 @@ void push_counters(Map* m)
 		c.bbox[3 + i] = 0ull;
 	}
 	*m->h_ctr = c;
-	CK(cudaMemcpyAsync(m->M.ctr, m->h_ctr, sizeof(Counters), cudaMemcpyHostToDevice, m->stream));
+	CK(cudaMemcpyAsync(m->M.ctr, m->h_ctr.get(), sizeof(Counters), cudaMemcpyHostToDevice, m->stream));
+}
+
+// grows the existing arrays of the brick pools (upper = false) or of the upper-node pool to the
+// capacities M holds now
+void grow_arrays(Map* m, bool upper)
+{
+	for_each_pool_array(m, [&](const PoolArray& a) {
+		if ((a.unit == Unit::kUpper) == upper && a.buf.get())
+			a.buf.grow(capacity(m->M, a.unit) * a.unit_bytes, a.fill, m->stream);
+	});
 }
 
 // grow whichever pool overflowed; `want_*` are the allocation counters the failed
@@ -292,7 +429,6 @@ void grow_pools(Map* m, uint32_t overflow, uint32_t want_bricks, uint32_t want_u
 {
 	DeviceMap& M = m->M;
 	cudaStream_t s = m->stream;
-	size_t& tot = m->device_bytes;
 	CK(cudaStreamSynchronize(s));
 	if (overflow & 2u) {
 		uint32_t oc = M.brick_cap;
@@ -300,38 +436,10 @@ void grow_pools(Map* m, uint32_t overflow, uint32_t want_bricks, uint32_t want_u
 		// capacity: small pools grow by 4x, large ones by 2x
 		uint32_t nc = (uint32_t)std::max<uint64_t>((oc < (1u << 18) ? 4ull : 2ull) * oc, (uint64_t)want_bricks + want_bricks / 4);
 		if ((uint64_t)nc * 64 > 0xfffffff0ull) throw std::bad_alloc();
-		const size_t ob = (size_t)oc * 64, nb = (size_t)nc * 64;
-		dev_grow(M.leaf, ob * 64, nb * 64, 0, s, tot);
-		dev_grow(M.miss_mask, ob, nb, 0, s, tot);
-		dev_grow(M.hit_mask, ob, nb, 0, s, tot);
-		dev_grow(M.chg_mask, ob, nb, 0, s, tot);
-		dev_grow(M.agg2, ob, nb, 0, s, tot);
-		dev_grow(M.meta, ob, nb, 0, s, tot);
-		dev_grow(M.sum1, ob * 8, nb * 8, 0, s, tot);
-		dev_grow(M.leaf_rgb, ob * 64, nb * 64, 0, s, tot);
-		dev_grow(M.sum1_rgb, ob * 8, nb * 8, 0, s, tot);
-		dev_grow(M.rgb2, ob, nb, 0, s, tot);
-		dev_grow(M.alias_miss, ob, nb, 0, s, tot);
-		dev_grow(M.alias_hit, ob, nb, 0, s, tot);
-		dev_grow(M.brick_key, oc, nc, 0, s, tot);
-		dev_grow(M.brick_stamp, oc, nc, 0, s, tot);
-		dev_grow(M.brick_parent, oc, nc, 0xff, s, tot);
-		dev_grow(M.touched, oc, nc, 0, s, tot);
-		dev_grow(M.touched_alt, oc, nc, 0, s, tot);
-		dev_grow(M.touched_mi, oc, nc, 0, s, tot);
-		dev_grow(M.touched_alt_mi, oc, nc, 0, s, tot);
-		dev_grow(M.brick_sum3, (size_t)oc * 8, (size_t)nc * 8, 0, s, tot);
-		dev_grow(M.brick_sum4, oc, nc, 0, s, tot);
-		dev_grow(M.brick_rgb3, (size_t)oc * 8, (size_t)nc * 8, 0, s, tot);
-		dev_grow(M.brick_rgb4, oc, nc, 0, s, tot);
 		M.brick_cap = nc;
+		grow_arrays(m, false);
 		// rebuild the hash from the surviving bricks (drops kFailed entries)
-		size_t old_tab = (size_t)M.bh_mask + 1;
-		uint32_t new_tab = std::max(kMinHash, next_pow2(2ull * nc));
-		CK(cudaFree(M.bh_tab));
-		tot -= old_tab * sizeof(ulonglong2);
-		M.bh_mask = new_tab - 1;
-		dev_alloc(M.bh_tab, new_tab, 0xff, s, tot);
+		alloc_brick_hash(m);
 		uint32_t live = std::min(m->h_ctr->n_bricks, oc);
 		if (live) k_rebuild_brick_hash<<<(live + 255) / 256, 256, 0, s>>>(M, live);
 		if (M.up_cap < nc / 2) overflow |= 4u;  // keep the upper-node pool in proportion
@@ -339,25 +447,9 @@ void grow_pools(Map* m, uint32_t overflow, uint32_t want_bricks, uint32_t want_u
 	if (overflow & 4u) {
 		uint32_t oc = M.up_cap;
 		uint32_t nc = (uint32_t)std::max<uint64_t>(std::max<uint64_t>(2ull * oc, M.brick_cap / 2), (uint64_t)want_upper + want_upper / 4);
-		dev_grow(M.up_key, oc, nc, 0, s, tot);
-		dev_grow(M.up_agg, oc, nc, 0, s, tot);
-		dev_grow(M.up_stamp, oc, nc, 0, s, tot);
-		dev_grow(M.up_rgb, oc, nc, 0, s, tot);
-		dev_grow(M.up_child, (size_t)oc * 8, (size_t)nc * 8, 0, s, tot);
-		dev_grow(M.up_child_rgb, (size_t)oc * 8, (size_t)nc * 8, 0, s, tot);
-		dev_grow(M.up_valid, oc, nc, 0, s, tot);
-		dev_grow(M.up_parent, oc, nc, 0xff, s, tot);
-		dev_grow(m->d_list[0], oc, nc, 0, s, tot);
-		dev_grow(m->d_list[1], oc, nc, 0, s, tot);
 		M.up_cap = nc;
-		size_t old_tab = (size_t)M.uh_mask + 1;
-		uint32_t new_tab = std::max(kMinHash, next_pow2(2ull * nc));
-		CK(cudaFree(M.uh_keys));
-		CK(cudaFree(M.uh_vals));
-		tot -= old_tab * (sizeof(unsigned long long) + sizeof(uint32_t));
-		M.uh_mask = new_tab - 1;
-		dev_alloc(M.uh_keys, new_tab, 0xff, s, tot);
-		dev_alloc(M.uh_vals, new_tab, 0xff, s, tot);
+		grow_arrays(m, true);
+		alloc_upper_hash(m);
 		uint32_t nu = std::min(m->h_ctr->n_upper, oc);
 		if (nu) k_rebuild_upper_hash<<<(nu + 255) / 256, 256, 0, s>>>(M, nu);
 	}
@@ -378,55 +470,31 @@ size_t layout_stride(int layout)
 // called with the stream idle
 void ensure_scan_buffers(Map* m, size_t n, bool need_table, bool records, bool fused)
 {
-	size_t& tot = m->device_bytes;
-	if (n > m->ray_cap) {
-		if (m->d_ray_end) {
-			cudaFree(m->d_ray_end);
-			cudaFree(m->d_hit_tab);
-			tot -= m->ray_cap * (3 * sizeof(double) + sizeof(uint32_t));
-		}
-		if (m->d_seg_base) {
-			cudaFree(m->d_seg_base);
-			cudaFree(m->d_seg_count);
-			cudaFree(m->d_order);
-			m->d_seg_base = m->d_seg_count = m->d_order = nullptr;
-			tot -= (m->ray_cap / 32 + 1) * 12;
-		}
-		size_t cap = std::max<size_t>(n, 1024);
-		dev_alloc(m->d_ray_end, cap * 3, 0, m->stream, tot);
-		dev_alloc(m->d_hit_tab, cap, 0xff, m->stream, tot);
-		m->ray_cap = cap;
+	cudaStream_t s = m->stream;
+	if (n > m->d_hit_tab.size()) {
+		m->d_seg_base.reset();  // sized by the ray capacity: allocated again below when needed
+		m->d_seg_count.reset();
+		m->d_order.reset();
+		const size_t cap = std::max<size_t>(n, 1024);
+		m->d_ray_end.resize(cap * 3, 0, s);
+		m->d_hit_tab.resize(cap, 0xff, s);
 	}
-	if (records && !m->d_seg_base) {
-		dev_alloc(m->d_seg_base, m->ray_cap / 32 + 1, 0, m->stream, tot);
-		dev_alloc(m->d_seg_count, m->ray_cap / 32 + 1, 0, m->stream, tot);
-		dev_alloc(m->d_order, m->ray_cap / 32 + 1, 0, m->stream, tot);
+	const size_t ray_cap = m->d_hit_tab.size();
+	if (records && !m->d_seg_base.get()) {
+		m->d_seg_base.resize(ray_cap / 32 + 1, 0, s);
+		m->d_seg_count.resize(ray_cap / 32 + 1, 0, s);
+		m->d_order.resize(ray_cap / 32 + 1, 0, s);
 	}
-	if (fused && m->item_cap < m->ray_cap) {
-		if (m->d_items) {
-			cudaFree(m->d_items);
-			cudaFree(m->d_vmask);
-			cudaFree(m->d_rc);
-			tot -= m->item_cap * (kShells * sizeof(Item) + sizeof(RayConst)) + (m->item_cap / 32 + 1) * kShells * 4;
-		}
-		m->item_cap = m->ray_cap;
-		m->d_items = nullptr;
-		CK(cudaMalloc(reinterpret_cast<void**>(&m->d_items), m->item_cap * kShells * sizeof(Item)));  // written before read
-		tot += m->item_cap * kShells * sizeof(Item);
-		dev_alloc(m->d_vmask, (m->item_cap / 32 + 1) * kShells, 0, m->stream, tot);
-		dev_alloc(m->d_rc, m->item_cap, 0, m->stream, tot);
+	if (fused && m->d_rc.size() < ray_cap) {
+		m->d_items.resize(ray_cap * kShells);  // written before read
+		m->d_vmask.resize((ray_cap / 32 + 1) * kShells, 0, s);
+		m->d_rc.resize(ray_cap, 0, s);
 	}
 	if (need_table) {
 		uint32_t want = std::max(1u << 12, next_pow2(4ull * n));
-		if (want > m->tab_size) {
-			if (m->d_tab_keys) {
-				cudaFree(m->d_tab_keys);
-				cudaFree(m->d_tab_min);
-				tot -= (size_t)m->tab_size * 12;
-			}
-			dev_alloc(m->d_tab_keys, want, 0xff, m->stream, tot);
-			dev_alloc(m->d_tab_min, want, 0xff, m->stream, tot);
-			m->tab_size = want;
+		if (want > m->d_tab_keys.size()) {
+			m->d_tab_keys.resize(want, 0xff, s);
+			m->d_tab_min.resize(want, 0xff, s);
 		}
 	}
 }
@@ -483,16 +551,9 @@ void finish_stats(Map* m)
 
 void ensure_seg(Map* m, unsigned long long want)
 {
-	if (want <= m->seg_cap) return;
+	if (want <= m->d_seg.size()) return;
 	CK(cudaStreamSynchronize(m->stream));
-	if (m->d_seg) {
-		cudaFree(m->d_seg);
-		m->device_bytes -= m->seg_cap * sizeof(QEntry);
-	}
-	m->d_seg = nullptr;
-	CK(cudaMalloc(reinterpret_cast<void**>(&m->d_seg), want * sizeof(QEntry)));
-	m->seg_cap = want;
-	m->device_bytes += want * sizeof(QEntry);
+	m->d_seg.resize(want);
 }
 
 // K3 over the scan's touched list: persistent warps, the list length is read on the device.
@@ -631,19 +692,13 @@ void setup_volume(Map* m, PendingScan& p, uint32_t db)
 {
 	DeviceMap& M = m->M;
 	if (db > m->vol_db_cap) {
-		if (M.vol) {
-			cudaFree(M.vol);
-			cudaFree(M.vol_dirty);
-			cudaFree(M.vol_list);
-			m->device_bytes -= (size_t)m->vol_db_cap * m->vol_db_cap * m->vol_db_cap * (512 + 1) ;
-		}
-		M.vol = nullptr;
-		M.vol_dirty = nullptr;
-		M.vol_list = nullptr;
 		const size_t nb = (size_t)db * db * db;
-		dev_alloc(M.vol, nb * 64, 0, m->stream, m->device_bytes);
-		dev_alloc(M.vol_dirty, nb / 64 + 1, 0, m->stream, m->device_bytes);
-		dev_alloc(M.vol_list, nb / 64 + 1, 0, m->stream, m->device_bytes);
+		m->vol.resize(nb * 64, 0, m->stream);
+		m->vol_dirty.resize(nb / 64 + 1, 0, m->stream);
+		m->vol_list.resize(nb / 64 + 1, 0, m->stream);
+		M.vol = m->vol.get();
+		M.vol_dirty = m->vol_dirty.get();
+		M.vol_list = m->vol_list.get();
 		m->vol_db_cap = db;
 	}
 	const Geometry& g = M.g;
@@ -653,6 +708,13 @@ void setup_volume(Map* m, PendingScan& p, uint32_t db)
 	M.vol_g0x = ((ko.x & 0x1fffffu) >> 4) - half;
 	M.vol_g0y = ((ko.y & 0x1fffffu) >> 4) - half;
 	M.vol_g0z = ((ko.z & 0x1fffffu) >> 4) - half;
+}
+
+// drops the marks left in the scan volume
+void wipe_volume(Map* m)
+{
+	m->vol.fill(0, m->stream);
+	m->vol_dirty.fill(0, m->stream);
 }
 
 // K4: upper levels, depth 5 .. L, from the touched list
@@ -710,36 +772,36 @@ void enqueue_scan(Map* m, PendingScan& p)
 	M.dense = (fused && p.dense) ? 1u : 0u;
 	M.mask_base = M.dense ? M.vol : M.miss_mask;
 	// (re-)bind the scan buffers: they may have been regrown since the scan was first enqueued
-	a.ray_end = m->d_ray_end;
-	a.tab_keys = m->d_tab_keys;
-	a.tab_min = m->d_tab_min;
-	a.tab_mask = m->tab_size ? m->tab_size - 1 : 0;
-	a.hit_tab = p.use_color ? m->d_hit_tab : nullptr;
+	a.ray_end = m->d_ray_end.get();
+	a.tab_keys = m->d_tab_keys.get();
+	a.tab_min = m->d_tab_min.get();
+	a.tab_mask = m->d_tab_keys.size() ? (uint32_t)m->d_tab_keys.size() - 1 : 0;
+	a.hit_tab = p.use_color ? m->d_hit_tab.get() : nullptr;
 	a.seg = nullptr;
 	a.seg_base = a.seg_count = a.order = nullptr;
 	a.items = nullptr;
 	if (fused) {
-		a.items = m->d_items;
-		a.item_stride = m->item_cap;
-		a.vmask = m->d_vmask;
-		a.rc = m->d_rc;
+		a.items = m->d_items.get();
+		a.item_stride = m->d_rc.size();
+		a.vmask = m->d_vmask.get();
+		a.rc = m->d_rc.get();
 	} else if (!p.simple && !p.has_vol) {
-		a.seg = m->d_seg;
-		a.seg_cap = m->seg_cap;
-		a.seg_base = m->d_seg_base;
-		a.seg_count = m->d_seg_count;
-		a.order = m->d_order;
+		a.seg = m->d_seg.get();
+		a.seg_cap = m->d_seg.size();
+		a.seg_base = m->d_seg_base.get();
+		a.seg_count = m->d_seg_count.get();
+		a.order = m->d_order.get();
 	}
 	if (a.depth >= 5) {
-		if (!m->d_nodes) dev_alloc(m->d_nodes, (size_t)1 << 20, 0, s, m->device_bytes);
-		a.nodes = m->d_nodes;
+		if (!m->d_nodes.get()) m->d_nodes.resize((size_t)1 << 20, 0, s);
+		a.nodes = m->d_nodes.get();
 		a.nodes_cap = 1u << 20;
 	}
 	m->ev7_valid = false;
 	push_counters(m);
 	if (p.need_table) {
-		CK(cudaMemsetAsync(m->d_tab_keys, 0xff, (size_t)m->tab_size * sizeof(unsigned long long), s));
-		CK(cudaMemsetAsync(m->d_tab_min, 0xff, (size_t)m->tab_size * sizeof(uint32_t), s));
+		m->d_tab_keys.fill(0xff, s);
+		m->d_tab_min.fill(0xff, s);
 	}
 	if (p.has_vol) {
 		// setValueVolume: the marks come from the box instead of a scan
@@ -782,7 +844,7 @@ void enqueue_scan(Map* m, PendingScan& p)
 	launch_upper(m);
 	CK(cudaEventRecord(m->ev[6], s));
 	m->ev_valid = true;
-	CK(cudaMemcpyAsync(m->h_ctr, M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
+	CK(cudaMemcpyAsync(m->h_ctr.get(), M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
 	m->stats_pending = true;
 	p.valid = true;
 }
@@ -799,7 +861,7 @@ void finalize_scan(Map* m)
 	}
 	DeviceMap& M = m->M;
 	if (p.routed) {
-		const uint32_t rf = m->h_route_flag ? *m->h_route_flag : 0u;
+		const uint32_t rf = m->h_route_flag.get() ? *m->h_route_flag : 0u;
 		if (rf || (m->route_stage == 1 && m->h_ctr->overflow)) {
 			if (rf) m->set_error("routed mode: an inbox region is too small (flags %u); raise cap_bricks / cap_hits", rf);
 			else m->set_error("routed mode: a device pool overflowed while marking (flags %u); create the map with a larger initial_bricks", m->h_ctr->overflow);
@@ -834,7 +896,7 @@ void finalize_scan(Map* m)
 				k_reset_upper_pass<<<1, 1, 0, m->stream>>>(M.ctr, nu);
 				launch_upper(m);
 				CK(cudaEventRecord(m->ev[6], m->stream));
-				CK(cudaMemcpyAsync(m->h_ctr, M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, m->stream));
+				CK(cudaMemcpyAsync(m->h_ctr.get(), M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, m->stream));
 			} else {
 				// an allocation failed while marking: nothing was consumed (K3/K4 backed off).  Grow,
 				// keep the bricks that were created, and run the whole scan again under a new scan id
@@ -845,22 +907,15 @@ void finalize_scan(Map* m)
 					// as a safety net): wipe the volume and repeat through the brick hash
 					m->no_dense = 1;
 					p.dense = false;
-					const size_t nb = (size_t)m->vol_db_cap * m->vol_db_cap * m->vol_db_cap;
-					CK(cudaMemsetAsync(M.vol, 0, nb * 512, m->stream));
-					CK(cudaMemsetAsync(M.vol_dirty, 0, (nb / 64 + 1) * 8, m->stream));
+					wipe_volume(m);
 				}
 				if (ov & 32u) {
 					// first out-of-tree key ever seen by this map: allocate the alias mask arrays;
 					// from now on this map uses the generic record path
-					if (!M.alias_miss) {
-						dev_alloc(M.alias_miss, (size_t)M.brick_cap * 64, 0, m->stream, m->device_bytes);
-						dev_alloc(M.alias_hit, (size_t)M.brick_cap * 64, 0, m->stream, m->device_bytes);
-					}
+					alloc_arrays(m, Exists::kAlias);
 					if (p.dense) {
 						// the marks the walk already left in the volume are not consumed by the record path
-						const size_t nb = (size_t)m->vol_db_cap * m->vol_db_cap * m->vol_db_cap;
-						CK(cudaMemsetAsync(M.vol, 0, nb * 512, m->stream));
-						CK(cudaMemsetAsync(M.vol_dirty, 0, (nb / 64 + 1) * 8, m->stream));
+						wipe_volume(m);
 						p.dense = false;
 					}
 				}
@@ -951,6 +1006,21 @@ int sync_map(Map* m)
 	return UFO_B200_OK;
 }
 
+// Starts the copy of a host cloud to the device, on the copy stream, into the staging buffer the
+// scan in flight is not using: the H2D copy of scan k+1 overlaps the kernels of scan k (the
+// reference overlaps its own front end with the previous scan's helper thread the same way,
+// OMB:315).  Returns where the scan reads the points.
+const void* stage_points(Map* m, const void* points, size_t bytes)
+{
+	m->stage ^= 1u;
+	Buffer<unsigned char>& buf = m->d_points[m->stage];
+	if (bytes > buf.size()) buf.resize(std::max<size_t>(bytes + bytes / 8, 1 << 16));
+	CK(cudaEventRecord(m->ev_copy0, m->copy_stream));
+	CK(cudaMemcpyAsync(buf.get(), points, bytes, cudaMemcpyHostToDevice, m->copy_stream));
+	CK(cudaEventRecord(m->ev_copied, m->copy_stream));
+	return buf.get();
+}
+
 int do_insert(Map* m, const double origin[3], const void* points, bool on_device, size_t n,
               const double* frame_pose,
               int layout, double max_range, uint32_t depth, int simple, uint32_t early_stopping,
@@ -991,27 +1061,10 @@ int do_insert(Map* m, const double origin[3], const void* points, bool on_device
 	}
 	CK(cudaSetDevice(m->device));
 
-	// The points go to the device first, on the copy stream, into the staging buffer the scan in
-	// flight is not using: the H2D copy of scan k+1 overlaps the kernels of scan k (the reference
-	// overlaps its own front end with the previous scan's helper thread the same way, OMB:315).
+	// an on-device cloud is read in place: it has to stay valid until the scan is done
 	const size_t bytes = n * stride;
 	const bool copied = !on_device && bytes;
-	const uint32_t stg = m->stage ^ 1u;
-	if (copied) {
-		if (bytes > m->d_points_cap[stg]) {
-			if (m->d_points[stg]) {
-				cudaFree(m->d_points[stg]);
-				m->device_bytes -= m->d_points_cap[stg];
-			}
-			m->d_points[stg] = nullptr;
-			m->d_points_cap[stg] = std::max<size_t>(bytes + bytes / 8, 1 << 16);
-			CK(cudaMalloc(&m->d_points[stg], m->d_points_cap[stg]));
-			m->device_bytes += m->d_points_cap[stg];
-		}
-		CK(cudaEventRecord(m->ev_copy0, m->copy_stream));
-		CK(cudaMemcpyAsync(m->d_points[stg], points, bytes, cudaMemcpyHostToDevice, m->copy_stream));
-		CK(cudaEventRecord(m->ev_copied, m->copy_stream));
-	}
+	const void* src = copied ? stage_points(m, points, bytes) : points;
 	// one integration in flight at most (insertPointCloudWait, occupancy_map_base.h:315)
 	finalize_scan(m);
 
@@ -1061,11 +1114,9 @@ int do_insert(Map* m, const double origin[3], const void* points, bool on_device
 	}
 	if (records) {
 		// first guess for the record buffer: 48 records per ray; grown on demand
-		ensure_seg(m, std::max<unsigned long long>(m->seg_cap, std::max<unsigned long long>(n, 1024) * 48ull));
+		ensure_seg(m, std::max<unsigned long long>(m->d_seg.size(), std::max<unsigned long long>(n, 1024) * 48ull));
 	}
-	// an on-device cloud is read in place: it has to stay valid until the scan is done
-	a.points = on_device ? points : m->d_points[stg];
-	if (copied) m->stage = stg;
+	a.points = src;
 
 	m->stats = ufo_b200_scan_stats{};
 	m->stats.points = n;
@@ -1105,7 +1156,7 @@ void route_fill_table(Map* m)
 		T.out[r].hdr = reinterpret_cast<uint32_t*>(bo);
 		T.out[r].miss = reinterpret_cast<unsigned long long*>(bo + m->route_miss_off);
 		T.out[r].hit = reinterpret_cast<unsigned long long*>(bo + m->route_hit_off);
-		unsigned char* bi = m->route_inbox + ((size_t)m->route_parity * W + r) * m->route_region;
+		unsigned char* bi = m->route_inbox.get() + ((size_t)m->route_parity * W + r) * m->route_region;
 		T.in[r].hdr = reinterpret_cast<uint32_t*>(bi);
 		T.in[r].miss = reinterpret_cast<unsigned long long*>(bi + m->route_miss_off);
 		T.in[r].hit = reinterpret_cast<unsigned long long*>(bi + m->route_hit_off);
@@ -1131,22 +1182,7 @@ int do_route_mark(Map* m, const double origin[3], const void* points, bool on_de
 	CK(cudaSetDevice(m->device));
 	const size_t bytes = n * stride;
 	const bool copied = !on_device && bytes;
-	const uint32_t stg = m->stage ^ 1u;
-	if (copied) {
-		if (bytes > m->d_points_cap[stg]) {
-			if (m->d_points[stg]) {
-				cudaFree(m->d_points[stg]);
-				m->device_bytes -= m->d_points_cap[stg];
-			}
-			m->d_points[stg] = nullptr;
-			m->d_points_cap[stg] = std::max<size_t>(bytes + bytes / 8, 1 << 16);
-			CK(cudaMalloc(&m->d_points[stg], m->d_points_cap[stg]));
-			m->device_bytes += m->d_points_cap[stg];
-		}
-		CK(cudaEventRecord(m->ev_copy0, m->copy_stream));
-		CK(cudaMemcpyAsync(m->d_points[stg], points, bytes, cudaMemcpyHostToDevice, m->copy_stream));
-		CK(cudaEventRecord(m->ev_copied, m->copy_stream));
-	}
+	const void* src = copied ? stage_points(m, points, bytes) : points;
 	finalize_scan(m);
 	cudaStream_t s = m->stream;
 	PendingScan& p = m->pending;
@@ -1167,13 +1203,12 @@ int do_route_mark(Map* m, const double origin[3], const void* points, bool on_de
 	}
 	M.dense = p.dense ? 1u : 0u;
 	M.mask_base = M.dense ? M.vol : M.miss_mask;
-	a.points = on_device ? points : m->d_points[stg];
-	if (copied) m->stage = stg;
-	a.ray_end = m->d_ray_end;
-	a.items = m->d_items;
-	a.item_stride = m->item_cap;
-	a.vmask = m->d_vmask;
-	a.rc = m->d_rc;
+	a.points = src;
+	a.ray_end = m->d_ray_end.get();
+	a.items = m->d_items.get();
+	a.item_stride = m->d_rc.size();
+	a.vmask = m->d_vmask.get();
+	a.rc = m->d_rc.get();
 	m->stats = ufo_b200_scan_stats{};
 	m->stats.points = n;
 	m->launches = 0;
@@ -1184,7 +1219,7 @@ int do_route_mark(Map* m, const double origin[3], const void* points, bool on_de
 	route_fill_table(m);
 	*m->h_route_flag = 0;
 	CK(cudaEventRecord(m->ev[0], s));
-	CK(cudaMemcpyAsync(M.route, m->h_route, sizeof(RouteTable), cudaMemcpyHostToDevice, s));
+	CK(cudaMemcpyAsync(M.route, m->h_route.get(), sizeof(RouteTable), cudaMemcpyHostToDevice, s));
 	if (copied) CK(cudaStreamWaitEvent(s, m->ev_copied, 0));
 	M.scan_id += 1;
 	if (M.scan_id == 0) M.scan_id = 1;
@@ -1202,8 +1237,8 @@ int do_route_mark(Map* m, const double origin[3], const void* points, bool on_de
 	m->launches += 2;
 	if (m->profiling) CK(cudaEventRecord(m->ev[3], s));
 	CK(cudaGetLastError());
-	CK(cudaMemcpyAsync(m->h_route_flag, &M.route->overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-	CK(cudaMemcpyAsync(m->h_ctr, M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
+	CK(cudaMemcpyAsync(m->h_route_flag.get(), &M.route->overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+	CK(cudaMemcpyAsync(m->h_ctr.get(), M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
 	p.valid = true;
 	m->route_stage = 1;
 	if (copied) CK(cudaEventSynchronize(m->ev_copied));
@@ -1246,7 +1281,7 @@ int do_route_apply(Map* m, uint32_t first, uint32_t count, int last)
 		launch_upper_levels(m);
 		CK(cudaEventRecord(m->ev[6], s));
 		m->ev_valid = true;
-		CK(cudaMemcpyAsync(m->h_ctr, M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
+		CK(cudaMemcpyAsync(m->h_ctr.get(), M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
 		m->stats_pending = true;
 		m->route_stage = 2;
 	}
@@ -1272,6 +1307,49 @@ int guarded(Map* m, F&& f)
 		if (m) m->set_error("out of memory");
 		return UFO_B200_E_NOMEM;
 	}
+}
+
+// Copies the first k entries of a device result list back to the caller's arrays (null ones are
+// skipped); colours are packed r | g << 8 | b << 16 on the device, 3 bytes on the host.  Waits for s.
+void copy_results(cudaStream_t s, size_t k, const unsigned long long* d_codes, uint64_t* codes, const float* d_occ,
+                  float* logodds, const uint32_t* d_rgb, uint8_t* rgb)
+{
+	if (codes) CK(cudaMemcpyAsync(codes, d_codes, k * 8, cudaMemcpyDeviceToHost, s));
+	if (logodds) CK(cudaMemcpyAsync(logodds, d_occ, k * 4, cudaMemcpyDeviceToHost, s));
+	std::vector<uint32_t> h(rgb ? k : 0);
+	if (rgb) CK(cudaMemcpyAsync(h.data(), d_rgb, k * 4, cudaMemcpyDeviceToHost, s));
+	CK(cudaStreamSynchronize(s));
+	for (size_t i = 0; i < h.size(); ++i) {
+		rgb[3 * i] = h[i] & 0xff;
+		rgb[3 * i + 1] = (h[i] >> 8) & 0xff;
+		rgb[3 * i + 2] = (h[i] >> 16) & 0xff;
+	}
+}
+
+// launch(codes, occ, rgb, cap, count) enqueues kernels that count results into count and write the
+// first cap of them to the lists (cap is 0 while the caller asks for the count only).  *n = the
+// count; what fits in the caller's arrays is copied back.
+template <class Launch>
+void collect_results(Map* m, uint64_t* codes, float* logodds, uint8_t* rgb, size_t cap, size_t* n, Launch&& launch)
+{
+	cudaStream_t s = m->stream;
+	const bool fill = codes != nullptr && cap > 0;
+	Buffer<unsigned long long> d_count, d_codes;
+	Buffer<float> d_occ;
+	Buffer<uint32_t> d_rgb;
+	d_count.resize(1, 0, s);
+	if (fill) {
+		d_codes.resize(cap);
+		d_occ.resize(cap);
+		if (rgb) d_rgb.resize(cap);
+	}
+	launch(d_codes.get(), d_occ.get(), d_rgb.get(), fill ? cap : 0, d_count.get());
+	CK(cudaGetLastError());
+	unsigned long long cnt = 0;
+	CK(cudaMemcpyAsync(&cnt, d_count.get(), 8, cudaMemcpyDeviceToHost, s));
+	CK(cudaStreamSynchronize(s));
+	*n = (size_t)cnt;
+	if (fill) copy_results(s, std::min<size_t>(cnt, cap), d_codes.get(), codes, d_occ.get(), logodds, d_rgb.get(), rgb);
 }
 }  // namespace
 
@@ -1350,7 +1428,7 @@ int ufo_b200_create(const ufo_b200_params* p, ufo_b200_map** out)
 		CK(cudaEventCreate(&m->ev_copied));
 		m->stream = m->own_stream;
 		for (auto& e : m->ev) CK(cudaEventCreate(&e));
-		CK(cudaHostAlloc(reinterpret_cast<void**>(&m->h_ctr), sizeof(Counters), cudaHostAllocDefault));
+		m->h_ctr.resize(1);
 		m->M.g = make_geometry(p->resolution, p->depth_levels);
 		m->M.color = p->color ? 1u : 0u;
 		m->M.shard_rank = 0;
@@ -1378,8 +1456,7 @@ int ufo_b200_create(const ufo_b200_params* p, ufo_b200_map** out)
 	});
 	if (rc != UFO_B200_OK) {
 		fprintf(stderr, "ufo_b200_create failed: %s\n", m->err.c_str());
-		free_pools(m);
-		delete m;
+		ufo_b200_destroy(m);
 		return rc;
 	}
 	*out = m;
@@ -1389,22 +1466,10 @@ int ufo_b200_create(const ufo_b200_params* p, ufo_b200_map** out)
 void ufo_b200_destroy(ufo_b200_map* m)
 {
 	if (!m) return;
-	if (m->device == -2) {
-		delete m;
-		return;
+	if (m->device != -2) {
+		cudaSetDevice(m->device);
+		cudaStreamSynchronize(m->stream);
 	}
-	cudaSetDevice(m->device);
-	cudaStreamSynchronize(m->stream);
-	free_pools(m);
-	for (auto& e : m->ev)
-		if (e) cudaEventDestroy(e);
-	if (m->h_ctr) cudaFreeHost(m->h_ctr);
-	if (m->h_route) cudaFreeHost(m->h_route);
-	if (m->h_route_flag) cudaFreeHost(m->h_route_flag);
-	if (m->own_stream) cudaStreamDestroy(m->own_stream);
-	if (m->copy_stream) cudaStreamDestroy(m->copy_stream);
-	if (m->ev_copy0) cudaEventDestroy(m->ev_copy0);
-	if (m->ev_copied) cudaEventDestroy(m->ev_copied);
 	delete m;
 }
 
@@ -1624,38 +1689,22 @@ int ufo_b200_query(ufo_b200_map* m, const uint64_t* codes, const uint32_t* depth
 		CK(cudaSetDevice(m->device));
 		sync_map(m);
 		cudaStream_t s = m->stream;
-		unsigned long long* d_codes = nullptr;
-		uint32_t *d_depths = nullptr, *d_rgb = nullptr;
-		float* d_occ = nullptr;
-		uint8_t* d_flags = nullptr;
-		CK(cudaMalloc(&d_codes, n * 8));
-		CK(cudaMalloc(&d_depths, n * 4));
-		CK(cudaMalloc(&d_occ, n * 4));
-		CK(cudaMalloc(&d_flags, n));
-		if (rgb) CK(cudaMalloc(&d_rgb, n * 4));
-		CK(cudaMemcpyAsync(d_codes, codes, n * 8, cudaMemcpyHostToDevice, s));
-		CK(cudaMemcpyAsync(d_depths, depths, n * 4, cudaMemcpyHostToDevice, s));
-		k_query<<<(uint32_t)((n + 255) / 256), 256, 0, s>>>(m->M, d_codes, d_depths, (uint32_t)n, d_occ, d_flags, d_rgb);
+		Buffer<unsigned long long> d_codes;
+		Buffer<uint32_t> d_depths, d_rgb;
+		Buffer<float> d_occ;
+		Buffer<uint8_t> d_flags;
+		d_codes.resize(n);
+		d_depths.resize(n);
+		d_occ.resize(n);
+		d_flags.resize(n);
+		if (rgb) d_rgb.resize(n);
+		CK(cudaMemcpyAsync(d_codes.get(), codes, n * 8, cudaMemcpyHostToDevice, s));
+		CK(cudaMemcpyAsync(d_depths.get(), depths, n * 4, cudaMemcpyHostToDevice, s));
+		k_query<<<(uint32_t)((n + 255) / 256), 256, 0, s>>>(m->M, d_codes.get(), d_depths.get(), (uint32_t)n, d_occ.get(),
+		                                                    d_flags.get(), d_rgb.get());
 		CK(cudaGetLastError());
-		CK(cudaMemcpyAsync(logodds, d_occ, n * 4, cudaMemcpyDeviceToHost, s));
-		CK(cudaMemcpyAsync(flags, d_flags, n, cudaMemcpyDeviceToHost, s));
-		std::vector<uint32_t> h_rgb;
-		if (rgb) {
-			h_rgb.resize(n);
-			CK(cudaMemcpyAsync(h_rgb.data(), d_rgb, n * 4, cudaMemcpyDeviceToHost, s));
-		}
-		CK(cudaStreamSynchronize(s));
-		if (rgb)
-			for (size_t i = 0; i < n; ++i) {
-				rgb[3 * i] = h_rgb[i] & 0xff;
-				rgb[3 * i + 1] = (h_rgb[i] >> 8) & 0xff;
-				rgb[3 * i + 2] = (h_rgb[i] >> 16) & 0xff;
-			}
-		cudaFree(d_codes);
-		cudaFree(d_depths);
-		cudaFree(d_occ);
-		cudaFree(d_flags);
-		if (d_rgb) cudaFree(d_rgb);
+		CK(cudaMemcpyAsync(flags, d_flags.get(), n, cudaMemcpyDeviceToHost, s));
+		copy_results(s, n, nullptr, nullptr, d_occ.get(), logodds, d_rgb.get(), rgb);
 		return (int)UFO_B200_OK;
 	});
 }
@@ -1667,45 +1716,12 @@ int ufo_b200_export_leaves(ufo_b200_map* m, uint64_t* codes, float* logodds, uin
 	return guarded(m, [&]() {
 		CK(cudaSetDevice(m->device));
 		sync_map(m);
-		cudaStream_t s = m->stream;
-		unsigned long long* d_count = nullptr;
-		CK(cudaMalloc(&d_count, 8));
-		CK(cudaMemsetAsync(d_count, 0, 8, s));
-		unsigned long long* d_codes = nullptr;
-		float* d_occ = nullptr;
-		uint32_t* d_rgb = nullptr;
-		bool fill = codes != nullptr && cap > 0;
-		if (fill) {
-			CK(cudaMalloc(&d_codes, cap * 8));
-			CK(cudaMalloc(&d_occ, cap * 4));
-			if (rgb) CK(cudaMalloc(&d_rgb, cap * 4));
-		}
-		size_t threads = (size_t)m->n_bricks * 64 * 64;
-		if (threads)
-			k_export<<<(uint32_t)((threads + 255) / 256), 256, 0, s>>>(m->M, m->n_bricks, d_codes, d_occ, d_rgb, fill ? cap : 0, d_count);
-		CK(cudaGetLastError());
-		unsigned long long cnt = 0;
-		CK(cudaMemcpyAsync(&cnt, d_count, 8, cudaMemcpyDeviceToHost, s));
-		CK(cudaStreamSynchronize(s));
-		*n = (size_t)cnt;
-		if (fill) {
-			size_t k = std::min<size_t>(cnt, cap);
-			CK(cudaMemcpy(codes, d_codes, k * 8, cudaMemcpyDeviceToHost));
-			if (logodds) CK(cudaMemcpy(logodds, d_occ, k * 4, cudaMemcpyDeviceToHost));
-			if (rgb) {
-				std::vector<uint32_t> h(k);
-				CK(cudaMemcpy(h.data(), d_rgb, k * 4, cudaMemcpyDeviceToHost));
-				for (size_t i = 0; i < k; ++i) {
-					rgb[3 * i] = h[i] & 0xff;
-					rgb[3 * i + 1] = (h[i] >> 8) & 0xff;
-					rgb[3 * i + 2] = (h[i] >> 16) & 0xff;
-				}
-			}
-			cudaFree(d_codes);
-			cudaFree(d_occ);
-			if (d_rgb) cudaFree(d_rgb);
-		}
-		cudaFree(d_count);
+		collect_results(m, codes, logodds, rgb, cap, n, [&](unsigned long long* d_codes, float* d_occ, uint32_t* d_rgb,
+		                                                     size_t d_cap, unsigned long long* d_count) {
+			const size_t threads = (size_t)m->n_bricks * 64 * 64;
+			if (threads)
+				k_export<<<(uint32_t)((threads + 255) / 256), 256, 0, m->stream>>>(m->M, m->n_bricks, d_codes, d_occ, d_rgb, d_cap, d_count);
+		});
 		return (int)UFO_B200_OK;
 	});
 }
@@ -1900,93 +1916,82 @@ int export_image(Map* m, int pruned, uint32_t min_depth, const double* box6, boo
 	}
 	plan.info.resize(nb);
 	std::vector<unsigned long long> keys(nb);
-	BrickInfo* d_info = nullptr;
-	unsigned long long* d_offs = nullptr;
-	uint8_t* d_out = nullptr;
-	auto cleanup = [&]() {
-		if (d_info) cudaFree(d_info);
-		if (d_offs) cudaFree(d_offs);
-		if (d_out) cudaFree(d_out);
-	};
-	try {
-		if (nb) {
-			CK(cudaMalloc(&d_info, sizeof(BrickInfo) * nb));
-			if (color) k_brick_stream<true><<<nb, 64, 0, s>>>(m->M, nb, pruned, min_depth, plan.box, d_info, nullptr, nullptr);
-			else k_brick_stream<false><<<nb, 64, 0, s>>>(m->M, nb, pruned, min_depth, plan.box, d_info, nullptr, nullptr);
-			CK(cudaGetLastError());
-			CK(cudaMemcpyAsync(plan.info.data(), d_info, sizeof(BrickInfo) * nb, cudaMemcpyDeviceToHost, s));
-			CK(cudaMemcpyAsync(keys.data(), m->M.brick_key, 8ull * nb, cudaMemcpyDeviceToHost, s));
-			CK(cudaStreamSynchronize(s));
-		}
-		// bricks that are part of the tree, in Morton order; a leaf brick with the default payload is
-		// indistinguishable from untouched space
-		std::vector<std::pair<unsigned long long, uint32_t>> sorted;
-		sorted.reserve(nb);
-		for (uint32_t b = 0; b < nb; ++b) {
-			const BrickInfo& bi = plan.info[b];
-			if (bi.flags & 2u) continue;
-			if (!(bi.flags & 1u) && bi.occ == 0.0f && bi.rgb == 0u) continue;
-			uint32_t x, y, z;
-			unpack_key(keys[b], x, y, z);
-			sorted.emplace_back(spread3_host(x) | (spread3_host(y) << 1) | (spread3_host(z) << 2), b);
-		}
-		std::sort(sorted.begin(), sorted.end());
-		plan.order.resize(sorted.size());
-		plan.codes.resize(sorted.size());
-		std::vector<unsigned long long> offs(nb, ~0ull);
-		unsigned long long packed_bytes = 0;
-		for (size_t i = 0; i < sorted.size(); ++i) {
-			plan.codes[i] = sorted[i].first;
-			plan.order[i] = sorted[i].second;
-			const BrickInfo& bi = plan.info[sorted[i].second];
-			if (bi.flags & 4u) {
-				offs[sorted[i].second] = packed_bytes;
-				packed_bytes += bi.size;
-			}
-		}
-		bool root_has = false;
-		unsigned long long data_size = 1 + plan.P;  // children byte + root payload
-		if (!sorted.empty()) {
-			build_upper(plan, plan.levels, 0, sorted.size(), c0);
-			root_has = plan.nodes[0].has;
-			if (root_has) data_size = 1 + plan.nodes[0].size;
-		}
-		std::vector<uint8_t> packed(packed_bytes);
-		if (packed_bytes) {
-			CK(cudaMalloc(&d_offs, 8ull * nb));
-			CK(cudaMalloc(&d_out, packed_bytes));
-			CK(cudaMemcpyAsync(d_offs, offs.data(), 8ull * nb, cudaMemcpyHostToDevice, s));
-			if (color) k_brick_stream<true><<<nb, 64, kBrickStreamMax, s>>>(m->M, nb, pruned, min_depth, plan.box, d_info, d_offs, d_out);
-			else k_brick_stream<false><<<nb, 64, kBrickStreamMax, s>>>(m->M, nb, pruned, min_depth, plan.box, d_info, d_offs, d_out);
-			CK(cudaGetLastError());
-			CK(cudaMemcpyAsync(packed.data(), d_out, packed_bytes, cudaMemcpyDeviceToHost, s));
-			CK(cudaStreamSynchronize(s));
-		}
-		unsigned long long produced = 0;
-		auto counted = [&](const void* p, size_t len) {
-			sink(p, len);
-			produced += len;
-		};
-		if (with_header) {
-			char head[512];
-			const int hl = header(head, sizeof head, data_size);
-			counted(head, (size_t)hl);
-		}
-		const uint8_t children = root_has ? 0xff : 0x00;
-		counted(&children, 1);
-		if (root_has) {
-			emit_upper(plan, offs, packed.data(), 0, plan.levels, counted);
-		} else {
-			const float occ = sorted.empty() ? 0.0f : plan.nodes[0].occ;
-			const uint32_t rgb = sorted.empty() ? 0u : plan.nodes[0].rgb;
-			put_payload_host(counted, plan.P, occ, rgb);
-		}
-		*total = produced;
-	} catch (...) {
-		cleanup();
-		throw;
+	Buffer<BrickInfo> d_info;
+	Buffer<unsigned long long> d_offs;
+	Buffer<uint8_t> d_out;
+	if (nb) {
+		d_info.resize(nb);
+		if (color) k_brick_stream<true><<<nb, 64, 0, s>>>(m->M, nb, pruned, min_depth, plan.box, d_info.get(), nullptr, nullptr);
+		else k_brick_stream<false><<<nb, 64, 0, s>>>(m->M, nb, pruned, min_depth, plan.box, d_info.get(), nullptr, nullptr);
+		CK(cudaGetLastError());
+		CK(cudaMemcpyAsync(plan.info.data(), d_info.get(), sizeof(BrickInfo) * nb, cudaMemcpyDeviceToHost, s));
+		CK(cudaMemcpyAsync(keys.data(), m->M.brick_key, 8ull * nb, cudaMemcpyDeviceToHost, s));
+		CK(cudaStreamSynchronize(s));
 	}
-	cleanup();
+	// bricks that are part of the tree, in Morton order; a leaf brick with the default payload is
+	// indistinguishable from untouched space
+	std::vector<std::pair<unsigned long long, uint32_t>> sorted;
+	sorted.reserve(nb);
+	for (uint32_t b = 0; b < nb; ++b) {
+		const BrickInfo& bi = plan.info[b];
+		if (bi.flags & 2u) continue;
+		if (!(bi.flags & 1u) && bi.occ == 0.0f && bi.rgb == 0u) continue;
+		uint32_t x, y, z;
+		unpack_key(keys[b], x, y, z);
+		sorted.emplace_back(spread3_host(x) | (spread3_host(y) << 1) | (spread3_host(z) << 2), b);
+	}
+	std::sort(sorted.begin(), sorted.end());
+	plan.order.resize(sorted.size());
+	plan.codes.resize(sorted.size());
+	std::vector<unsigned long long> offs(nb, ~0ull);
+	unsigned long long packed_bytes = 0;
+	for (size_t i = 0; i < sorted.size(); ++i) {
+		plan.codes[i] = sorted[i].first;
+		plan.order[i] = sorted[i].second;
+		const BrickInfo& bi = plan.info[sorted[i].second];
+		if (bi.flags & 4u) {
+			offs[sorted[i].second] = packed_bytes;
+			packed_bytes += bi.size;
+		}
+	}
+	bool root_has = false;
+	unsigned long long data_size = 1 + plan.P;  // children byte + root payload
+	if (!sorted.empty()) {
+		build_upper(plan, plan.levels, 0, sorted.size(), c0);
+		root_has = plan.nodes[0].has;
+		if (root_has) data_size = 1 + plan.nodes[0].size;
+	}
+	std::vector<uint8_t> packed(packed_bytes);
+	if (packed_bytes) {
+		d_offs.resize(nb);
+		d_out.resize(packed_bytes);
+		CK(cudaMemcpyAsync(d_offs.get(), offs.data(), 8ull * nb, cudaMemcpyHostToDevice, s));
+		if (color) k_brick_stream<true><<<nb, 64, kBrickStreamMax, s>>>(m->M, nb, pruned, min_depth, plan.box, d_info.get(), d_offs.get(), d_out.get());
+		else k_brick_stream<false><<<nb, 64, kBrickStreamMax, s>>>(m->M, nb, pruned, min_depth, plan.box, d_info.get(), d_offs.get(), d_out.get());
+		CK(cudaGetLastError());
+		CK(cudaMemcpyAsync(packed.data(), d_out.get(), packed_bytes, cudaMemcpyDeviceToHost, s));
+		CK(cudaStreamSynchronize(s));
+	}
+	unsigned long long produced = 0;
+	auto counted = [&](const void* p, size_t len) {
+		sink(p, len);
+		produced += len;
+	};
+	if (with_header) {
+		char head[512];
+		const int hl = header(head, sizeof head, data_size);
+		counted(head, (size_t)hl);
+	}
+	const uint8_t children = root_has ? 0xff : 0x00;
+	counted(&children, 1);
+	if (root_has) {
+		emit_upper(plan, offs, packed.data(), 0, plan.levels, counted);
+	} else {
+		const float occ = sorted.empty() ? 0.0f : plan.nodes[0].occ;
+		const uint32_t rgb = sorted.empty() ? 0u : plan.nodes[0].rgb;
+		put_payload_host(counted, plan.P, occ, rgb);
+	}
+	*total = produced;
 	return UFO_B200_OK;
 }
 }  // namespace
@@ -2270,31 +2275,13 @@ int ufo_b200_clear(ufo_b200_map* m)
 		}
 		DeviceMap& M = m->M;
 		cudaStream_t s = m->stream;
-		CK(cudaMemsetAsync(M.bh_tab, 0xff, ((size_t)M.bh_mask + 1) * sizeof(ulonglong2), s));
-		CK(cudaMemsetAsync(M.uh_keys, 0xff, ((size_t)M.uh_mask + 1) * 8, s));
-		CK(cudaMemsetAsync(M.uh_vals, 0xff, ((size_t)M.uh_mask + 1) * 4, s));
-		CK(cudaMemsetAsync(M.brick_stamp, 0, (size_t)m->n_bricks * 4, s));
-		CK(cudaMemsetAsync(M.up_stamp, 0, (size_t)m->n_upper * 4, s));
-		CK(cudaMemsetAsync(M.up_valid, 0, (size_t)m->n_upper * 4, s));
-		CK(cudaMemsetAsync(M.up_parent, 0xff, (size_t)m->n_upper * 4, s));
-		CK(cudaMemsetAsync(M.brick_parent, 0xff, (size_t)m->n_bricks * 4, s));
-		const size_t nb = (size_t)m->n_bricks * 64;
-		CK(cudaMemsetAsync(M.leaf, 0, nb * 64 * 4, s));
-		CK(cudaMemsetAsync(M.miss_mask, 0, nb * 8, s));
-		CK(cudaMemsetAsync(M.hit_mask, 0, nb * 8, s));
-		CK(cudaMemsetAsync(M.agg2, 0, nb * sizeof(Agg), s));
-		CK(cudaMemsetAsync(M.meta, 0, nb * 4, s));
-		if (M.color) CK(cudaMemsetAsync(M.leaf_rgb, 0, nb * 64 * 4, s));
-		if (M.alias_miss) {
-			CK(cudaMemsetAsync(M.alias_miss, 0, nb * 8, s));
-			CK(cudaMemsetAsync(M.alias_hit, 0, nb * 8, s));
-		}
-		if (M.chg_mask) CK(cudaMemsetAsync(M.chg_mask, 0, nb * 8, s));
-		if (M.vol) {
-			const size_t vb = (size_t)m->vol_db_cap * m->vol_db_cap * m->vol_db_cap;
-			CK(cudaMemsetAsync(M.vol, 0, vb * 512, s));
-			CK(cudaMemsetAsync(M.vol_dirty, 0, (vb / 64 + 1) * 8, s));
-		}
+		m->bh_tab.fill(0xff, s);
+		m->uh_keys.fill(0xff, s);
+		m->uh_vals.fill(0xff, s);
+		for_each_pool_array(m, [&](const PoolArray& a) {
+			if (a.cleared && a.buf.get()) a.buf.fill(a.fill, s, in_use(m, a.unit) * a.unit_bytes);
+		});
+		if (m->vol.get()) wipe_volume(m);
 		m->n_blocks = 0;
 		m->n_bricks = 0;
 		m->n_upper = 0;
@@ -2338,24 +2325,22 @@ int ufo_b200_route_setup(ufo_b200_map* m, uint32_t rank, uint32_t world, uint32_
 	return guarded(m, [&]() {
 		CK(cudaSetDevice(m->device));
 		sync_map(m);
-		if (m->n_bricks != 0 || m->route_inbox || m->M.shard_world > 1 || m->M.color) {
+		if (m->n_bricks != 0 || m->route_inbox.get() || m->M.shard_world > 1 || m->M.color) {
 			m->set_error("ufo_b200_route_setup: needs an empty, unsharded mono map and may be called once");
 			return (int)UFO_B200_E_INVALID;
 		}
 		const size_t total = route_layout(world, cap_bricks, cap_hits, &m->route_region, &m->route_miss_off, &m->route_hit_off);
-		CK(cudaMalloc(reinterpret_cast<void**>(&m->route_inbox), total));
-		CK(cudaMemset(m->route_inbox, 0, total));
-		CK(cudaMalloc(reinterpret_cast<void**>(&m->M.route), sizeof(RouteTable)));
-		CK(cudaMemset(m->M.route, 0, sizeof(RouteTable)));
-		CK(cudaHostAlloc(reinterpret_cast<void**>(&m->h_route), sizeof(RouteTable), cudaHostAllocDefault));
-		CK(cudaHostAlloc(reinterpret_cast<void**>(&m->h_route_flag), sizeof(uint32_t), cudaHostAllocDefault));
+		m->route_inbox.resize(total, 0);
+		m->route.resize(1, 0);
+		m->M.route = m->route.get();
+		m->h_route.resize(1);
+		m->h_route_flag.resize(1);
 		*m->h_route_flag = 0;
-		m->device_bytes += total + sizeof(RouteTable);
 		m->route_cap_m = cap_bricks;
 		m->route_cap_h = cap_hits;
 		m->M.route_rank = rank;
 		m->M.route_world = world;
-		*inbox = m->route_inbox;
+		*inbox = m->route_inbox.get();
 		return (int)UFO_B200_OK;
 	});
 }
@@ -2412,20 +2397,13 @@ int ufo_b200_enable_change_detection(ufo_b200_map* m, int enable)
 	return guarded(m, [&]() {
 		CK(cudaSetDevice(m->device));
 		sync_map(m);
-		DeviceMap& M = m->M;
-		if (enable && !M.chg_mask) {
-			dev_alloc(M.chg_mask, (size_t)M.brick_cap * 64, 0, m->stream, m->device_bytes);
+		// the mask is allocated by the first enable and kept: switched off, it keeps the recorded set
+		m->chg_recording = enable != 0;
+		if (enable && !m->chg_mask) {
+			alloc_arrays(m, Exists::kChange);
 			CK(cudaStreamSynchronize(m->stream));
-		} else if (!enable && M.chg_mask) {
-			// the reference keeps the recorded set when detection is switched off; so do we: the
-			// mask array stays, recording stops
-			m->chg_paused = M.chg_mask;
-			M.chg_mask = nullptr;
 		}
-		if (enable && !M.chg_mask && m->chg_paused) {
-			M.chg_mask = m->chg_paused;
-			m->chg_paused = nullptr;
-		}
+		m->M.chg_mask = m->chg_recording ? m->chg_mask : nullptr;
 		return (int)UFO_B200_OK;
 	});
 }
@@ -2436,8 +2414,9 @@ int ufo_b200_reset_change_detection(ufo_b200_map* m)
 	return guarded(m, [&]() {
 		CK(cudaSetDevice(m->device));
 		sync_map(m);
-		unsigned long long* p = m->M.chg_mask ? m->M.chg_mask : m->chg_paused;
-		if (p) CK(cudaMemsetAsync(p, 0, (size_t)m->M.brick_cap * 64 * 8, m->stream));
+		for_each_pool_array(m, [&](const PoolArray& a) {
+			if (a.exists == Exists::kChange && a.buf.get()) a.buf.fill(0, m->stream);
+		});
 		return (int)UFO_B200_OK;
 	});
 }
@@ -2450,47 +2429,36 @@ int ufo_b200_changed_codes(ufo_b200_map* m, uint32_t depth, uint64_t* codes, siz
 		sync_map(m);
 		*n = 0;
 		DeviceMap M = m->M;
-		if (!M.chg_mask) M.chg_mask = m->chg_paused;
+		M.chg_mask = m->chg_mask;  // also while recording is switched off
 		if (!M.chg_mask || !m->n_bricks) return (int)UFO_B200_OK;
 		if (depth > M.g.depth_levels) return (int)UFO_B200_E_INVALID;
 		const uint32_t dd = std::min(depth, 4u);
 		cudaStream_t s = m->stream;
-		unsigned long long *d_count = nullptr, *d_codes = nullptr;
-		CK(cudaMalloc(&d_count, 8));
-		auto cleanup = [&]() {
-			if (d_count) cudaFree(d_count);
-			if (d_codes) cudaFree(d_codes);
-		};
-		try {
-			const uint32_t grid = (uint32_t)(((size_t)m->n_bricks * 64 + 255) / 256);
-			CK(cudaMemsetAsync(d_count, 0, 8, s));
-			k_changed<<<grid, 256, 0, s>>>(M, m->n_bricks, dd, nullptr, 0, d_count);
-			unsigned long long cnt = 0;
-			CK(cudaMemcpyAsync(&cnt, d_count, 8, cudaMemcpyDeviceToHost, s));
+		Buffer<unsigned long long> d_count, d_codes;
+		d_count.resize(1, 0, s);
+		const uint32_t grid = (uint32_t)(((size_t)m->n_bricks * 64 + 255) / 256);
+		k_changed<<<grid, 256, 0, s>>>(M, m->n_bricks, dd, nullptr, 0, d_count.get());
+		unsigned long long cnt = 0;
+		CK(cudaMemcpyAsync(&cnt, d_count.get(), 8, cudaMemcpyDeviceToHost, s));
+		CK(cudaStreamSynchronize(s));
+		std::vector<unsigned long long> h(cnt);
+		if (cnt) {
+			d_codes.resize(cnt);
+			d_count.fill(0, s);
+			k_changed<<<grid, 256, 0, s>>>(M, m->n_bricks, dd, d_codes.get(), cnt, d_count.get());
+			CK(cudaMemcpyAsync(h.data(), d_codes.get(), cnt * 8, cudaMemcpyDeviceToHost, s));
 			CK(cudaStreamSynchronize(s));
-			std::vector<unsigned long long> h(cnt);
-			if (cnt) {
-				CK(cudaMalloc(&d_codes, cnt * 8));
-				CK(cudaMemsetAsync(d_count, 0, 8, s));
-				k_changed<<<grid, 256, 0, s>>>(M, m->n_bricks, dd, d_codes, cnt, d_count);
-				CK(cudaMemcpyAsync(h.data(), d_codes, cnt * 8, cudaMemcpyDeviceToHost, s));
-				CK(cudaStreamSynchronize(s));
-			}
-			if (depth >= 4) {
-				// ancestors above the brick + duplicates: snap to `depth` (with the centre bits) and unique
-				const unsigned long long lowmask = depth >= 21 ? ~0ull : ((1ull << (3 * depth)) - 1ull);
-				const unsigned long long centre = key_to_code({1u << (depth - 1), 1u << (depth - 1), 1u << (depth - 1)});
-				for (auto& c : h) c = (c & ~lowmask) | centre;
-				std::sort(h.begin(), h.end());
-				h.erase(std::unique(h.begin(), h.end()), h.end());
-			}
-			*n = h.size();
-			if (codes) std::memcpy(codes, h.data(), std::min(cap, h.size()) * 8);
-		} catch (...) {
-			cleanup();
-			throw;
 		}
-		cleanup();
+		if (depth >= 4) {
+			// ancestors above the brick + duplicates: snap to `depth` (with the centre bits) and unique
+			const unsigned long long lowmask = depth >= 21 ? ~0ull : ((1ull << (3 * depth)) - 1ull);
+			const unsigned long long centre = key_to_code({1u << (depth - 1), 1u << (depth - 1), 1u << (depth - 1)});
+			for (auto& c : h) c = (c & ~lowmask) | centre;
+			std::sort(h.begin(), h.end());
+			h.erase(std::unique(h.begin(), h.end()), h.end());
+		}
+		*n = h.size();
+		if (codes) std::memcpy(codes, h.data(), std::min(cap, h.size()) * 8);
 		return (int)UFO_B200_OK;
 	});
 }
@@ -2557,29 +2525,19 @@ int ufo_b200_cast_rays(ufo_b200_map* m, const double* origins, const double* dir
 				rays[6 * i + 3 + k] = directions[3 * i + k];
 			}
 		}
-		double* d_rays = nullptr;
-		unsigned long long* d_codes = nullptr;
-		uint8_t* d_hit = nullptr;
-		auto cleanup = [&]() {
-			if (d_rays) cudaFree(d_rays);
-			if (d_codes) cudaFree(d_codes);
-			if (d_hit) cudaFree(d_hit);
-		};
-		try {
-			CK(cudaMalloc(&d_rays, rays.size() * 8));
-			CK(cudaMalloc(&d_codes, n * 8));
-			CK(cudaMalloc(&d_hit, n));
-			CK(cudaMemcpyAsync(d_rays, rays.data(), rays.size() * 8, cudaMemcpyHostToDevice, s));
-			k_cast_rays<<<(uint32_t)((n + 127) / 128), 128, 0, s>>>(m->M, d_rays, (uint32_t)n, ignore_unknown, max_range, depth, d_codes, d_hit);
-			CK(cudaGetLastError());
-			CK(cudaMemcpyAsync(codes, d_codes, n * 8, cudaMemcpyDeviceToHost, s));
-			CK(cudaMemcpyAsync(hit, d_hit, n, cudaMemcpyDeviceToHost, s));
-			CK(cudaStreamSynchronize(s));
-		} catch (...) {
-			cleanup();
-			throw;
-		}
-		cleanup();
+		Buffer<double> d_rays;
+		Buffer<unsigned long long> d_codes;
+		Buffer<uint8_t> d_hit;
+		d_rays.resize(rays.size());
+		d_codes.resize(n);
+		d_hit.resize(n);
+		CK(cudaMemcpyAsync(d_rays.get(), rays.data(), rays.size() * 8, cudaMemcpyHostToDevice, s));
+		k_cast_rays<<<(uint32_t)((n + 127) / 128), 128, 0, s>>>(m->M, d_rays.get(), (uint32_t)n, ignore_unknown, max_range, depth,
+		                                                        d_codes.get(), d_hit.get());
+		CK(cudaGetLastError());
+		CK(cudaMemcpyAsync(codes, d_codes.get(), n * 8, cudaMemcpyDeviceToHost, s));
+		CK(cudaMemcpyAsync(hit, d_hit.get(), n, cudaMemcpyDeviceToHost, s));
+		CK(cudaStreamSynchronize(s));
 		return (int)UFO_B200_OK;
 	});
 }
@@ -2605,53 +2563,15 @@ int ufo_b200_export_nodes(ufo_b200_map* m, uint32_t depth, int occupied, int fre
 				f.box.hi[k] = box6[k] + box6[3 + k];
 			}
 		}
-		cudaStream_t s = m->stream;
-		unsigned long long *d_count = nullptr, *d_codes = nullptr;
-		float* d_occ = nullptr;
-		uint32_t* d_rgb = nullptr;
-		auto cleanup = [&]() {
-			for (void* p : {(void*)d_count, (void*)d_codes, (void*)d_occ, (void*)d_rgb})
-				if (p) cudaFree(p);
-		};
-		try {
-			CK(cudaMalloc(&d_count, 8));
-			const bool fill = codes != nullptr && cap > 0;
-			if (fill) {
-				CK(cudaMalloc(&d_codes, cap * 8));
-				CK(cudaMalloc(&d_occ, cap * 4));
-				if (rgb) CK(cudaMalloc(&d_rgb, cap * 4));
-			}
-			CK(cudaMemsetAsync(d_count, 0, 8, s));
+		collect_results(m, codes, logodds, rgb, cap, n, [&](unsigned long long* d_codes, float* d_occ, uint32_t* d_rgb,
+		                                                     size_t d_cap, unsigned long long* d_count) {
 			if (depth <= 4) {
 				const size_t threads = (size_t)m->n_bricks * 64;
-				if (threads) k_export_nodes<<<(uint32_t)((threads + 255) / 256), 256, 0, s>>>(m->M, m->n_bricks, f, d_codes, d_occ, d_rgb, fill ? cap : 0, d_count);
+				if (threads) k_export_nodes<<<(uint32_t)((threads + 255) / 256), 256, 0, m->stream>>>(m->M, m->n_bricks, f, d_codes, d_occ, d_rgb, d_cap, d_count);
 			} else if (m->n_upper) {
-				k_export_upper<<<(m->n_upper + 255) / 256, 256, 0, s>>>(m->M, m->n_upper, f, d_codes, d_occ, d_rgb, fill ? cap : 0, d_count);
+				k_export_upper<<<(m->n_upper + 255) / 256, 256, 0, m->stream>>>(m->M, m->n_upper, f, d_codes, d_occ, d_rgb, d_cap, d_count);
 			}
-			CK(cudaGetLastError());
-			unsigned long long cnt = 0;
-			CK(cudaMemcpyAsync(&cnt, d_count, 8, cudaMemcpyDeviceToHost, s));
-			CK(cudaStreamSynchronize(s));
-			*n = (size_t)cnt;
-			if (fill) {
-				const size_t k = std::min<size_t>(cnt, cap);
-				CK(cudaMemcpy(codes, d_codes, k * 8, cudaMemcpyDeviceToHost));
-				if (logodds) CK(cudaMemcpy(logodds, d_occ, k * 4, cudaMemcpyDeviceToHost));
-				if (rgb) {
-					std::vector<uint32_t> h(k);
-					CK(cudaMemcpy(h.data(), d_rgb, k * 4, cudaMemcpyDeviceToHost));
-					for (size_t i = 0; i < k; ++i) {
-						rgb[3 * i] = h[i] & 0xff;
-						rgb[3 * i + 1] = (h[i] >> 8) & 0xff;
-						rgb[3 * i + 2] = (h[i] >> 16) & 0xff;
-					}
-				}
-			}
-		} catch (...) {
-			cleanup();
-			throw;
-		}
-		cleanup();
+		});
 		return (int)UFO_B200_OK;
 	});
 }
@@ -2802,60 +2722,49 @@ int import_stream(Map* m, const uint8_t* data, size_t size, const double* box6)
 	// the codes of a tree of L levels use 3L bits; the pools must hold the bricks the stream creates
 	cudaStream_t s = m->stream;
 	const size_t n_small = plan.small.size(), n_bricks = plan.bricks.size(), n_wipe = plan.wipe.size();
-	ImportRec *d_small = nullptr, *d_bricks = nullptr, *d_wipe = nullptr;
-	auto cleanup = [&]() {
-		for (void* p : {(void*)d_small, (void*)d_bricks, (void*)d_wipe})
-			if (p) cudaFree(p);
-	};
-	try {
-		if (n_small) {
-			CK(cudaMalloc(&d_small, n_small * sizeof(ImportRec)));
-			CK(cudaMemcpyAsync(d_small, plan.small.data(), n_small * sizeof(ImportRec), cudaMemcpyHostToDevice, s));
-		}
-		if (n_bricks) {
-			CK(cudaMalloc(&d_bricks, n_bricks * sizeof(ImportRec)));
-			CK(cudaMemcpyAsync(d_bricks, plan.bricks.data(), n_bricks * sizeof(ImportRec), cudaMemcpyHostToDevice, s));
-		}
-		if (n_wipe) {
-			CK(cudaMalloc(&d_wipe, n_wipe * sizeof(ImportRec)));
-			CK(cudaMemcpyAsync(d_wipe, plan.wipe.data(), n_wipe * sizeof(ImportRec), cudaMemcpyHostToDevice, s));
-		}
-		for (int attempt = 0;; ++attempt) {
-			M.scan_id++;
-			if (M.scan_id == 0) M.scan_id = 1;
-			M.up_epoch++;
-			M.dense = 0;
-			M.mask_base = M.miss_mask;
-			push_counters(m);
-			if (n_wipe && m->n_bricks)
-				k_import_wipe<<<(uint32_t)(((size_t)m->n_bricks * 64 + 255) / 256), 256, 0, s>>>(M, m->n_bricks, d_wipe, (uint32_t)n_wipe);
-			if (n_bricks) k_import_bricks<<<(uint32_t)std::min<size_t>(n_bricks, (size_t)m->sm_count * 16), 64, 0, s>>>(M, d_bricks, (uint32_t)n_bricks);
-			if (n_small) k_import_small<<<m->sm_count * 8, 256, 0, s>>>(M, d_small, (uint32_t)n_small);
-			k_import_refresh<<<m->sm_count * 8, 256, 0, s>>>(M);
-			if (M.color) k_brick_agg<true><<<m->sm_count * 4, 256, 0, s>>>(M);
-			else k_brick_agg<false><<<m->sm_count * 4, 256, 0, s>>>(M);
-			launch_upper(m);
-			CK(cudaGetLastError());
-			CK(cudaMemcpyAsync(m->h_ctr, M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
-			CK(cudaStreamSynchronize(s));
-			const uint32_t ov = m->h_ctr->overflow;
-			if (!ov) break;
-			if (attempt > 16) {
-				m->set_error("readData: device pools keep overflowing");
-				cleanup();
-				return UFO_B200_E_NOMEM;
-			}
-			// writing leaves is idempotent: grow and run the whole import again
-			m->n_bricks = std::min(m->h_ctr->n_bricks, M.brick_cap);
-			grow_pools(m, ov & 6u, m->h_ctr->n_bricks, m->h_ctr->n_upper);
-		}
-		m->n_bricks = std::min(m->h_ctr->n_bricks, M.brick_cap);
-		m->n_upper = std::min(m->h_ctr->n_upper, M.up_cap);
-	} catch (...) {
-		cleanup();
-		throw;
+	Buffer<ImportRec> d_small, d_bricks, d_wipe;
+	if (n_small) {
+		d_small.resize(n_small);
+		CK(cudaMemcpyAsync(d_small.get(), plan.small.data(), n_small * sizeof(ImportRec), cudaMemcpyHostToDevice, s));
 	}
-	cleanup();
+	if (n_bricks) {
+		d_bricks.resize(n_bricks);
+		CK(cudaMemcpyAsync(d_bricks.get(), plan.bricks.data(), n_bricks * sizeof(ImportRec), cudaMemcpyHostToDevice, s));
+	}
+	if (n_wipe) {
+		d_wipe.resize(n_wipe);
+		CK(cudaMemcpyAsync(d_wipe.get(), plan.wipe.data(), n_wipe * sizeof(ImportRec), cudaMemcpyHostToDevice, s));
+	}
+	for (int attempt = 0;; ++attempt) {
+		M.scan_id++;
+		if (M.scan_id == 0) M.scan_id = 1;
+		M.up_epoch++;
+		M.dense = 0;
+		M.mask_base = M.miss_mask;
+		push_counters(m);
+		if (n_wipe && m->n_bricks)
+			k_import_wipe<<<(uint32_t)(((size_t)m->n_bricks * 64 + 255) / 256), 256, 0, s>>>(M, m->n_bricks, d_wipe.get(), (uint32_t)n_wipe);
+		if (n_bricks) k_import_bricks<<<(uint32_t)std::min<size_t>(n_bricks, (size_t)m->sm_count * 16), 64, 0, s>>>(M, d_bricks.get(), (uint32_t)n_bricks);
+		if (n_small) k_import_small<<<m->sm_count * 8, 256, 0, s>>>(M, d_small.get(), (uint32_t)n_small);
+		k_import_refresh<<<m->sm_count * 8, 256, 0, s>>>(M);
+		if (M.color) k_brick_agg<true><<<m->sm_count * 4, 256, 0, s>>>(M);
+		else k_brick_agg<false><<<m->sm_count * 4, 256, 0, s>>>(M);
+		launch_upper(m);
+		CK(cudaGetLastError());
+		CK(cudaMemcpyAsync(m->h_ctr.get(), M.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
+		CK(cudaStreamSynchronize(s));
+		const uint32_t ov = m->h_ctr->overflow;
+		if (!ov) break;
+		if (attempt > 16) {
+			m->set_error("readData: device pools keep overflowing");
+			return UFO_B200_E_NOMEM;
+		}
+		// writing leaves is idempotent: grow and run the whole import again
+		m->n_bricks = std::min(m->h_ctr->n_bricks, M.brick_cap);
+		grow_pools(m, ov & 6u, m->h_ctr->n_bricks, m->h_ctr->n_upper);
+	}
+	m->n_bricks = std::min(m->h_ctr->n_bricks, M.brick_cap);
+	m->n_upper = std::min(m->h_ctr->n_upper, M.up_cap);
 	return UFO_B200_OK;
 }
 }  // namespace
